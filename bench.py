@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3                 # ours: CUDA hot path, one process per GPU
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference --steps 2 --warmup 1          # reference arm: the CPU oracle port on the host cores
+    python bench.py ... --dump-outputs DIR                         # also write the last timed step's outputs to DIR/*.npy
 
 One step = student (CLIP-ViT-6 + BERT-3/3, train mode incl. dropout) forward with KD outputs, teacher (ViT-12 + BERT-6/6)
 forward under no_grad, ITC / ITM / MLM losses, all KD losses (hidden + attention MSE with layer mapping, logit KL), backward,
@@ -590,22 +591,25 @@ def build_caption_infer(args, dev, rank, world):
             la.copy_((torch.randn(la.shape, generator=g) * 3.0 + args.loga_shift).to(dev))
     image = torch.randn(args.batch, 3, args.image_res, args.image_res, generator=torch.Generator().manual_seed(42 + rank))
     host = [image.pin_memory()]
+    outputs = {}        # what generate() hands its caller in the latest step (under a captured graph: the graph's output buffers)
 
     if args.beams > 1:
         # the decode the reference's evaluation runs (Eff_Captioning.py:201-202, Captioning.yaml: num_beams 3, max_length 20, min_length 5):
         # the beam scorer reads 2 * num_beams candidates per item back to the host every step, so this is an eager, host-driven loop
         def beam_step(image):
             _, ids = model.generate(image, sample=False, num_beams=args.beams, max_length=20, min_length=5, return_ids=True)
+            outputs["caption_ids"] = ids
             return ids.sum().float()
-        return dict(device_step=beam_step, host=host, optimizers=[], host_fn=None, units=args.batch, eager_only=True,
+        return dict(device_step=beam_step, host=host, optimizers=[], host_fn=None, units=args.batch, eager_only=True, outputs=outputs,
                     schedule="beam search (num_beams %d, max_length 20, min_length 5: transformers 4.12.5's algorithm restated, "
                              "BertLMHeadModel._beam_search): one decoder pass over batch x beams rows per token with a re-ordered KV cache, "
                              "one device -> host read per token for the hypothesis bookkeeping (not graph-capturable)" % args.beams)
 
     def device_step(image):
         _, ids = model.generate(image, greedy=True, max_length=20, return_ids=True, sync_free=not args.eager)
+        outputs["caption_ids"] = ids
         return ids.sum().float()
-    return dict(device_step=device_step, host=host, optimizers=[], host_fn=None, units=args.batch,
+    return dict(device_step=device_step, host=host, optimizers=[], host_fn=None, units=args.batch, outputs=outputs,
                 schedule="greedy decode loop of eff_bert.py:1472-1563 (one decoder pass per token, KV cache) run to max_length without the "
                          "per-token end-of-sequence check on the host (same ids; --eager keeps the check), so ViT + all decode steps are ONE "
                          "captured graph; the cross-attention K|V projections of the image tokens are computed once per caption batch")
@@ -634,6 +638,7 @@ def build_vqa_infer(args, dev, rank, world):
         n_before = sum(p.numel() for n, p in model.named_parameters() if not n.startswith("l0_module."))
         prune.materialize(model, zs)
         n_after = sum(p.numel() for n, p in model.named_parameters() if not n.startswith("l0_module."))
+    outputs = {}        # the ranked answers of the latest step (under a captured graph: the graph's output buffers)
 
     def device_step(image, q_ids, q_atts):
         with torch.no_grad():
@@ -641,6 +646,7 @@ def build_vqa_infer(args, dev, rank, world):
                 ids, probs, _ = model.fake_forward(image, Tok(q_ids, q_atts), Tok(l_ids, l_atts), k=128)
             else:
                 ids, probs = model(image, Tok(q_ids, q_atts), Tok(l_ids, l_atts), train=False, k=128)
+        outputs.update(answer_ids=ids, answer_probs=probs)
         return ids[:, 0].sum().float() + probs[:, 0].sum()     # one scalar that depends on every question's answer
 
     if args.materialize:
@@ -649,7 +655,7 @@ def build_vqa_infer(args, dev, rank, world):
                        n_before / 1e6, n_after / 1e6, kept_txt)
     else:
         schedule = "masked-dense: deterministic gates applied in the GEMM / attention epilogues (kept fraction per gate type: %s)" % kept_txt
-    return dict(device_step=device_step, host=host, optimizers=[], host_fn=None, units=args.batch,
+    return dict(device_step=device_step, host=host, optimizers=[], host_fn=None, units=args.batch, outputs=outputs,
                 schedule=schedule + "; candidates read their question through the cross-attention row index (no 128x tiling)")
 
 
@@ -855,6 +861,33 @@ def workload_text(args):
         args.image_res, args.batch)
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_ARENA_SAMPLE = 1 << 20     # parameter values kept per flat arena: 4 MB each, at most 12 arenas (three optimizers of four groups)
+
+
+def dump_outputs(out_dir, wl, last):
+    """Write what the timed path computed in its last step as `out_dir/<name>.npy` (floating data as float32, integers as float64), so
+    that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.  Inference workloads:
+    the arrays the model call returns.  Training steps: the loss the step returns and the parameters it updated, per flat arena of each
+    optimizer — whole up to DUMP_ARENA_SAMPLE values, else that many at indices drawn from a fixed seed (the same every run)."""
+    import numpy as np
+    arrays = dict(wl.get("outputs") or {"loss": last})
+    for i, opt in enumerate(wl["optimizers"]):
+        for j, g in enumerate(opt.param_groups):
+            p = g["p"]
+            if p.numel() > DUMP_ARENA_SAMPLE:
+                idx = torch.randint(p.numel(), (DUMP_ARENA_SAMPLE,), generator=torch.Generator().manual_seed(1000 * i + j)).sort().values
+                p = p[idx.to(p.device)]
+            arrays["params_opt%d_group%d" % (i, j)] = p
+    arrays = {k: v.detach().cpu() for k, v in arrays.items()}
+    arrays = {k: v.double() if (v.dtype == torch.float64 or not v.is_floating_point()) else v.float() for k, v in arrays.items()}
+    nbytes = sum(v.numel() * v.element_size() for v in arrays.values())
+    assert nbytes <= DUMP_MAX_BYTES, "--dump-outputs: %d bytes exceed the %d-byte limit" % (nbytes, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -888,7 +921,13 @@ def main():
     ap.add_argument("--eager", action="store_true", help="issue every launch from Python each step instead of replaying the captured step graph")
     ap.add_argument("--profile-step", action="store_true", help="warm up, then run ONE step between cudaProfilerStart/Stop and exit")
     ap.add_argument("--gemm-breakdown", action="store_true", help="print the per-shape GEMM time table to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last timed step computed "
+                    "(model outputs, or the loss and a fixed sample of the updated parameters) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.profile_step):
+        ap.error("--dump-outputs records the timed steps of --impl ours")
     metric, unit, def_batch, def_res, flop_per_unit = WORKLOADS[args.workload]
     args.batch = args.batch or def_batch
     args.image_res = args.image_res or def_res
@@ -922,10 +961,9 @@ def main():
         if rank != 0:
             return
         w = max(1, min(args.warmup, 1))
-        k = max(1, min(args.steps, 3))
+        k = args.steps
         v, med, threads = cpu_arm(k, w)
-        sample = "oracle port (CPU fp32, torch autograd), %d-unit sample of the same workload, %d timed steps (bounded from --steps %d)" % (
-            args.cpu_sample_batch, k, args.steps)
+        sample = "oracle port (CPU fp32, torch autograd), %d-unit sample of the same workload, %d timed steps" % (args.cpu_sample_batch, k)
         print(json.dumps({"impl": "reference", "metric": metric, "value": v, "unit": unit, "n_gpus": args.gpus, "steps": k,
                           "warmup": w, "ms_per_step": med * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                           "dtype": "f32", "data": "synthetic", "config": {"workload": workload, "sample_batch": args.cpu_sample_batch},
@@ -1059,6 +1097,8 @@ def main():
     if not (args.eager or args.profile_step):
         launches += graphed.captured_launches * args.steps      # ... plus the libevlm kernel nodes each replay executes
     host_enqueue_ms = host_ms[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl, last)      # before the end-to-end window's steps overwrite the outputs and parameters
     ms_e2e, last_e2e = timed(args.steps, True)
     if sampler:
         sampler.stop_flag = True

@@ -1,4 +1,4 @@
-"""Drop-in boundary test (CPU; needs the reference tree, skipped on the GPU box where /root/reference does not exist):
+"""Drop-in boundary test (CPU; needs a checkout of swaggy-TN/EfficientVLM named by $EVLM_REFERENCE_ROOT, skipped without one):
 the reference's OWN, unmodified task-model files (`efficient_models/model_{retrieval,generation,nlvr}.py`, `models/model_pretrain.py`)
 and the ITR driver's own `evaluation` / `itm_eval` functions (`Eff_Retrieval.py:216-378`) are imported on top of our
 `efficient_models.xvlm` / `models` packages (efficientvlm_b200/compat first on sys.path) and must reproduce the reference-generated
@@ -9,9 +9,10 @@ import sys
 
 import pytest
 
-REF = os.environ.get("EVLM_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("EVLM_REFERENCE_ROOT", "")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "efficient_models")), reason="reference tree not present")
+pytestmark = pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "efficient_models"))),
+                                reason="EVLM_REFERENCE_ROOT does not name a checkout of the reference code")
 
 SCRIPT = r'''
 import os, sys, types

@@ -203,7 +203,7 @@ def _worker(rank, world, port, q):
         q.put((rank, "FAIL: " + repr(e) + "\n" + traceback.format_exc()))
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs two GPUs")
 def test_two_gpu_nccl_step_matches_single_process():
     world = 2
     ctx = mp.get_context("spawn")
