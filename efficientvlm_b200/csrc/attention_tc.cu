@@ -281,7 +281,9 @@ __global__ void __launch_bounds__(TC_THREADS, 3) attn_fwd_tc_kernel(const __grid
         if (a.dropout_p > 0.f) {
 #pragma unroll
           for (int j = 0; j < 16; j += 4) {   // one Philox call per 4 consecutive keys (row stride padded to a multiple of 4)
-            const float4 u = dropout_uniform4(seed, a.dropout_stream, (erow + (uint64_t)(cc * 16 + j)) >> 2);
+            // the item's own key index (own-K/V pack: tile key - klo, a multiple of 4 since Lk % 8 == 0), so the mask does not
+            // depend on the pack slot; keys left of the row's block have P = 0 and are clamped rather than wrapped
+            const float4 u = dropout_uniform4(seed, a.dropout_stream, (erow + (uint64_t)max(cc * 16 + j - klo, 0)) >> 2);
             v[j] = u.x >= a.dropout_p ? v[j] * keep_inv : 0.f;
             v[j + 1] = u.y >= a.dropout_p ? v[j + 1] * keep_inv : 0.f;
             v[j + 2] = u.z >= a.dropout_p ? v[j + 2] * keep_inv : 0.f;

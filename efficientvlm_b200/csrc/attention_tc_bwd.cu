@@ -488,8 +488,9 @@ __global__ void __launch_bounds__(TB_THREADS, 1) attn_bwd_tc_kernel(const __grid
               const float4 m4 = *reinterpret_cast<const float4*>(mrow + ((j0 + j4) & MASK_AND));   // loaded per group of 4: 12 fewer live registers
               const float mk4[4] = {m4.x, m4.y, m4.z, m4.w};
               float dm[4] = {1.f, 1.f, 1.f, 1.f};
-              if (a.dropout_p > 0.f) {   // ONE Philox call per 4 consecutive keys (index = rowid * lkp4 + key)
-                const float4 u = dropout_uniform4(seed, a.dropout_stream, ((uint64_t)rowid * lkp4 + (uint64_t)(j0 + j4)) >> 2);
+              if (a.dropout_p > 0.f) {   // ONE Philox call per 4 consecutive keys (index = rowid * lkp4 + the item's own key)
+                // own-K/V pack: tile key - lo_me (keys left of the row's block have P = 0: clamped rather than wrapped), as the forward
+                const float4 u = dropout_uniform4(seed, a.dropout_stream, ((uint64_t)rowid * lkp4 + (uint64_t)max(j0 + j4 - lo_me, 0)) >> 2);
                 dm[0] = u.x >= a.dropout_p ? keep_inv : 0.f;
                 dm[1] = u.y >= a.dropout_p ? keep_inv : 0.f;
                 dm[2] = u.z >= a.dropout_p ? keep_inv : 0.f;
