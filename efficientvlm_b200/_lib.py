@@ -130,9 +130,14 @@ PROTOTYPES = {
     "evlm_index_add_rows": (c_i32, [c_p, c_p, c_p, c_i64, c_i64, c_p]),
     "evlm_index_fold_rows": (c_i32, [c_p, c_p, c_i64, c_i64, c_i64, c_p, c_p, c_p]),
     "evlm_rng_advance": (c_i32, [c_p, C.c_uint64, c_i32, c_p]),
+    "evlm_beam_step": (c_i32, [c_p, c_i64, c_i32, c_i32, c_i32, c_i32, c_i32, c_f, C.c_double, c_i32, c_i64, c_i64, c_p, c_i64, c_p, c_p, c_p,
+                               c_p, c_p, c_p, c_p, c_p, c_p]),
+    "evlm_beam_finalize": (c_i32, [c_p, c_i64, c_p, c_p, c_i32, c_i32, c_i32, c_i32, C.c_double, c_i64, c_i64, c_p, c_p, c_p, c_p, c_p, c_p,
+                                   c_p, c_p]),
+    "evlm_kv_beam_reorder": (c_i32, [C.POINTER(c_p), c_i32, c_i32, c_i32, c_i64, c_i64, c_i32, c_p, c_p]),
 }
 
-ABI_VERSION = 7   # must equal EVLM_ABI_VERSION in include/evlm.h
+ABI_VERSION = 8   # must equal EVLM_ABI_VERSION in include/evlm.h
 _lib = None
 
 

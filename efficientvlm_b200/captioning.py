@@ -98,8 +98,9 @@ class XVLMForCaptioning(XVLMBase):
     def generate(self, image, sample=False, num_beams=1, max_length=30, min_length=10, top_p=0.9, repetition_penalty=1.0,
                  num_return_sequences=1, greedy=False, return_ids=False, sync_free=False):
         """model_generation.py:407-484.  greedy / sample: the reference's own decode loop (`_generate_no_beam_search`); otherwise beam
-        search (`BertLMHeadModel._beam_search`: transformers 4.12.5's algorithm restated, parity unpinned).  return_ids=True (extension) also returns the generated token ids; sync_free=True
-        (extension) decodes to max_length without per-token host checks (same result, graph-capturable; see eff_bert)."""
+        search (`BertLMHeadModel.generate`: transformers 4.12.5's algorithm restated, parity unpinned; on CUDA the scorer runs on the device).
+        return_ids=True (extension) also returns the generated token ids; sync_free=True (extension) decodes to max_length without
+        host checks or reads (same result, graph-capturable; beam-search ids are then [batch, max_length], pad-filled; see eff_bert)."""
         zs = self._zs(False)
         vis_head = vis_mlp = None
         if zs is not None:
@@ -135,7 +136,7 @@ class XVLMForCaptioning(XVLMBase):
                           mlp_z=torch.cat((zs["text_intermediate_z"], zs["cross_intermediate_z"]), dim=0))
             outputs = self.text_decoder.generate(input_ids=input_ids, max_length=max_length, min_length=min_length, num_beams=num_beams,
                                                  eos_token_id=self.tokenizer.sep_token_id, pad_token_id=self.tokenizer.pad_token_id,
-                                                 repetition_penalty=repetition_penalty, **kw, **model_kwargs)
+                                                 repetition_penalty=repetition_penalty, sync_free=sync_free, **kw, **model_kwargs)
             captions = _get_captions(outputs)
             return (captions, outputs) if return_ids else captions
         if greedy:

@@ -18,6 +18,7 @@ from . import ops
 from ._lib import ACT_GELU_ERF
 from .eff_vit import find_pruneable_heads_and_indices, prune_linear_layer
 GREEDY_SELECT_FUSED = os.environ.get("EVLM_NO_GREEDY_FUSED") is None      # profiling knob: the framework's 17 small launches per token
+BEAM_SEARCH_ON_DEVICE = os.environ.get("EVLM_NO_DEVICE_BEAMS") is None    # beam search on CUDA tensors: device loop (off: the host loop)
 
 from .outputs import (BaseModelOutputWithPastAndCrossAttentions, BaseModelOutputWithPoolingAndCrossAttentions,
                       CausalLMOutputWithCrossAttentions, MaskedLMOutput)
@@ -750,20 +751,83 @@ class BertLMHeadModel(BertPreTrainedModel):
         return decoded
 
     @torch.no_grad()
+    def _beam_search_device(self, input_ids, num_beams, max_length, min_length, repetition_penalty, pad_token_id, eos_token_id,
+                            length_penalty=1.0, early_stopping=False, sync_free=False, **model_kwargs):
+        """`_beam_search` with the scorer on the device: every decode position is one decoder forward, one `evlm_beam_step` (log-softmax,
+        processors, top 2 * num_beams, BeamSearchScorer.process / BeamHypotheses bookkeeping) and one in-place `evlm_kv_beam_reorder` of
+        the self-attention caches; `evlm_beam_finalize` picks the results.  All state lives in device tensors and the loop runs exactly
+        max_length - prompt length steps with no device -> host read and no host -> device copy (finished items are frozen, so running
+        past the point where every item is done changes nothing).  sync_free=False returns the host loop's tensor (trimmed to the
+        output length with one read per call); sync_free=True returns [batch, max_length], pad after the output length, with no read at
+        all, so a caller can capture the whole call in one CUDA graph."""
+        batch, prompt_len = input_ids.shape
+        rows = batch * num_beams
+        dev = input_ids.device
+        enc = model_kwargs.get("encoder_hidden_states", None)
+        if enc is not None and not isinstance(enc, list) and enc.shape[0] != rows:
+            raise ValueError("encoder_hidden_states must hold batch * num_beams items (the caller expands them: model_generation.py:421-423)")
+        am = model_kwargs.pop("attention_mask", None)
+        if am is None:
+            mask = input_ids.new_ones((rows, max_length))     # the host loop's per-step `new_ones`, allocated once and sliced
+        else:
+            mask = am.new_ones((rows, max_length))
+            mask[:, :prompt_len] = am.repeat_interleave(num_beams, dim=0)
+        i32 = torch.int32
+        tokens = torch.full((rows, max_length), pad_token_id, dtype=torch.int64, device=dev)
+        tokens[:, :prompt_len] = input_ids.repeat_interleave(num_beams, dim=0)
+        beam_scores = torch.zeros(batch, num_beams, dtype=torch.float32, device=dev)
+        beam_scores[:, 1:] = -1e9
+        beam_scores = beam_scores.view(-1)
+        beam_src = torch.zeros(rows, dtype=i32, device=dev)
+        done = torch.zeros(batch, dtype=i32, device=dev)
+        hyp_tokens = torch.zeros(batch, num_beams, max_length, dtype=torch.int64, device=dev)
+        hyp_len = torch.zeros(batch, num_beams, dtype=i32, device=dev)
+        hyp_score = torch.zeros(batch, num_beams, dtype=torch.float64, device=dev)
+        hyp_count = torch.zeros(batch, dtype=i32, device=dev)
+        hyp_worst = torch.full((batch,), 1e9, dtype=torch.float64, device=dev)
+        item_base = None
+        past = None
+        for cur_len in range(prompt_len, max_length):
+            model_inputs = self.prepare_inputs_for_generation(tokens[:, :cur_len], past=past, attention_mask=mask[:, :cur_len], **model_kwargs)
+            outputs = self(**model_inputs, return_dict=True, use_cache=True)
+            past = outputs.past_key_values
+            K.beam_step(outputs.logits[:, -1, :].float(), num_beams, cur_len, min_length, repetition_penalty, length_penalty, early_stopping,
+                        eos_token_id, pad_token_id, tokens, beam_scores, beam_src, done, hyp_tokens, hyp_len, hyp_score, hyp_count, hyp_worst)
+            if cur_len + 1 < max_length and not ops.kv_beam_reorder(past, beam_src, num_beams):
+                if item_base is None:
+                    item_base = torch.arange(rows, device=dev) // num_beams * num_beams
+                past = self._reorder_cache(past, item_base + beam_src)
+        out, lengths = K.beam_finalize(num_beams, max_length, max_length, length_penalty, eos_token_id, pad_token_id, tokens, beam_scores, done,
+                                       hyp_tokens, hyp_len, hyp_score, hyp_count, hyp_worst)
+        if sync_free:
+            return out
+        return out[:, :min(int(lengths.max()) + 1, max_length)].contiguous()      # the call's one device -> host read
+
+    @torch.no_grad()
     def generate(self, input_ids, max_length=20, min_length=0, num_beams=1, do_sample=False, temperature=1.0, top_k=0, top_p=1.0,
-                 repetition_penalty=1.0, pad_token_id=0, eos_token_id=None, **model_kwargs):
-        """Greedy / sampling generation (num_beams == 1) through the in-repo loop; num_beams > 1: `_beam_search`, the algorithm the
-        reference's captioning evaluation gets from transformers 4.12.5's GenerationMixin (model_generation.py:474-483)."""
+                 repetition_penalty=1.0, pad_token_id=0, eos_token_id=None, sync_free=False, **model_kwargs):
+        """Greedy / sampling generation (num_beams == 1) through the in-repo loop; num_beams > 1: beam search, the algorithm the
+        reference's captioning evaluation gets from transformers 4.12.5's GenerationMixin (model_generation.py:474-483).  On CUDA tensors
+        (2 <= num_beams <= 8, a vocabulary above 2 * num_beams, at least one step to decode) it runs `_beam_search_device`, else the host
+        loop `_beam_search`.  sync_free=True (extension) runs every loop to max_length without host checks (same ids); beam search then
+        returns [batch, max_length] with pad after the output length."""
         if num_beams != 1:
             if do_sample:
                 raise NotImplementedError("beam sampling (num_beams > 1 with do_sample) is not used by the reference and not provided")
             if not isinstance(eos_token_id, int):
                 raise ValueError("beam search takes one end-of-sequence id (the reference passes tokenizer.sep_token_id)")
-            return self._beam_search(input_ids, num_beams, max_length, min_length, repetition_penalty, pad_token_id, eos_token_id,
-                                     **model_kwargs)
+            if (BEAM_SEARCH_ON_DEVICE and input_ids.is_cuda and 2 <= num_beams <= 8 and self.config.vocab_size > 2 * num_beams
+                    and input_ids.shape[1] < max_length):
+                return self._beam_search_device(input_ids, num_beams, max_length, min_length, repetition_penalty, pad_token_id, eos_token_id,
+                                                sync_free=sync_free, **model_kwargs)
+            ids = self._beam_search(input_ids, num_beams, max_length, min_length, repetition_penalty, pad_token_id, eos_token_id,
+                                    **model_kwargs)
+            if sync_free and ids.shape[1] < max_length:
+                ids = torch.cat([ids, ids.new_full((ids.shape[0], max_length - ids.shape[1]), pad_token_id)], dim=1)
+            return ids
         eos = [eos_token_id] if isinstance(eos_token_id, int) else list(eos_token_id or [])
         ids, _ = self._generate_no_beam_search(input_ids, input_ids.shape[1], max_length, do_sample, temperature, top_k, top_p,
-                                               repetition_penalty, pad_token_id, eos, input_ids.shape[0], **model_kwargs)
+                                               repetition_penalty, pad_token_id, eos, input_ids.shape[0], sync_free=sync_free, **model_kwargs)
         return ids
 
 

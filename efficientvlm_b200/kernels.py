@@ -733,6 +733,86 @@ def greedy_select(logits, unfinished, pad_token_id, eos_token_ids):
     return out[0], score, out[1], out[2]
 
 
+def _beam_check(cond, what, msg):
+    if not cond:
+        check(-1, "%s: %s" % (what, msg))
+
+
+def beam_step(logits, num_beams, cur_len, min_length, repetition_penalty, length_penalty, early_stopping, eos_token_id, pad_token_id,
+              tokens, beam_scores, beam_src, done, hyp_tokens, hyp_len, hyp_score, hyp_count, hyp_worst):
+    """One beam-search decode position for all items in one launch (include/evlm.h, evlm_beam_step).  logits fp32 [rows, vocab] with
+    rows = batch * num_beams (row pitch may exceed vocab); the loop state tensors are updated in place: tokens int64 [rows, width]
+    (history; column cur_len receives the new token), beam_scores fp32 [rows], beam_src int32 [rows], done int32 [batch], hyp_tokens
+    int64 [batch, num_beams, width], hyp_len int32 [batch, num_beams], hyp_score fp64 [batch, num_beams], hyp_count int32 [batch],
+    hyp_worst fp64 [batch]."""
+    what = "evlm_beam_step"
+    _beam_check(2 <= num_beams <= 8, what, "num_beams must be in 2..8")
+    _beam_check(logits.dtype == f32 and logits.dim() == 2 and logits.stride(1) == 1, what, "logits must be fp32 [rows, vocab] with unit stride")
+    rows, vocab = logits.shape
+    _beam_check(rows % num_beams == 0, what, "rows must be batch * num_beams")
+    batch = rows // num_beams
+    _beam_check(vocab > 2 * num_beams, what, "vocab must exceed 2 * num_beams")
+    _beam_check(tokens.dtype == torch.int64 and tokens.dim() == 2 and tokens.shape[0] == rows and tokens.is_contiguous(), what,
+                "tokens must be contiguous int64 [rows, width]")
+    width = tokens.shape[1]
+    _beam_check(1 <= cur_len < width, what, "cur_len must be inside the history width")
+    _beam_check(0 <= eos_token_id < vocab, what, "eos id outside the vocabulary")
+    _state_check(what, num_beams, batch, width, beam_scores, beam_src, done, hyp_tokens, hyp_len, hyp_score, hyp_count, hyp_worst)
+    check(_lib.load().evlm_beam_step(_p(logits), logits.stride(0), batch, num_beams, vocab, int(cur_len), int(min_length), float(repetition_penalty),
+                                     float(cur_len ** length_penalty), 1 if early_stopping else 0, int(eos_token_id), int(pad_token_id),
+                                     _p(tokens), width, _p(beam_scores), _p(beam_src), _p(done), _p(hyp_tokens), _p(hyp_len), _p(hyp_score),
+                                     _p(hyp_count), _p(hyp_worst), _stream()), what)
+
+
+def _state_check(what, num_beams, batch, width, beam_scores, beam_src, done, hyp_tokens, hyp_len, hyp_score, hyp_count, hyp_worst):
+    rows = batch * num_beams
+    for t, dt, shape in ((beam_scores, f32, (rows,)), (beam_src, torch.int32, (rows,)), (done, torch.int32, (batch,)),
+                         (hyp_tokens, torch.int64, (batch, num_beams, width)), (hyp_len, torch.int32, (batch, num_beams)),
+                         (hyp_score, torch.float64, (batch, num_beams)), (hyp_count, torch.int32, (batch,)), (hyp_worst, torch.float64, (batch,))):
+        if t is None:
+            continue
+        _beam_check(t.dtype == dt and tuple(t.shape) == shape and t.is_contiguous(), what, "beam state tensor must be contiguous %s %s" % (dt, shape))
+
+
+def beam_finalize(num_beams, cur_len, max_length, length_penalty, eos_token_id, pad_token_id, tokens, beam_scores, done, hyp_tokens, hyp_len,
+                  hyp_score, hyp_count, hyp_worst):
+    """BeamSearchScorer.finalize after the last step (history length cur_len).  Returns (out int64 [batch, max_length]: best hypothesis,
+    eos if shorter than max_length, pad; lengths int32 [batch])."""
+    what = "evlm_beam_finalize"
+    _beam_check(2 <= num_beams <= 8, what, "num_beams must be in 2..8")
+    _beam_check(tokens.dtype == torch.int64 and tokens.dim() == 2 and tokens.shape[0] % num_beams == 0 and tokens.is_contiguous(), what,
+                "tokens must be contiguous int64 [batch * num_beams, width]")
+    rows, width = tokens.shape
+    batch = rows // num_beams
+    _beam_check(1 <= cur_len <= width, what, "cur_len must be inside the history width")
+    _beam_check(1 <= max_length <= width, what, "max_length must not exceed the history width")
+    _state_check(what, num_beams, batch, width, beam_scores, None, done, hyp_tokens, hyp_len, hyp_score,
+                 hyp_count, hyp_worst)
+    out = torch.empty(batch, max_length, dtype=torch.int64, device=tokens.device)
+    lengths = torch.empty(batch, dtype=torch.int32, device=tokens.device)
+    check(_lib.load().evlm_beam_finalize(_p(tokens), width, _p(beam_scores), _p(done), batch, num_beams, int(cur_len), int(max_length),
+                                         float(cur_len ** length_penalty), int(eos_token_id), int(pad_token_id), _p(hyp_tokens), _p(hyp_len),
+                                         _p(hyp_score), _p(hyp_count), _p(hyp_worst), _p(out), _p(lengths), _stream()), what)
+    return out, lengths
+
+
+def kv_beam_reorder(caches, beam_src, num_beams, length):
+    """In place, ONE launch: for every cache (bf16 [batch * num_beams, capacity, row_elems], contiguous) and position < length, row r
+    takes the row of item(r) * num_beams + beam_src[r] (int32 [rows], 0 <= beam_src < num_beams)."""
+    what = "evlm_kv_beam_reorder"
+    _beam_check(2 <= num_beams <= 8, what, "num_beams must be in 2..8")
+    _beam_check(1 <= len(caches) <= 32, what, "1..32 caches")
+    shape = tuple(caches[0].shape)
+    _beam_check(len(shape) == 3 and shape[0] % num_beams == 0, what, "caches must be [batch * num_beams, capacity, row_elems]")
+    for c in caches:
+        _beam_check(c.dtype == bf16 and tuple(c.shape) == shape and c.is_contiguous(), what, "caches must be contiguous bf16 of one shape")
+    _beam_check(beam_src.dtype == torch.int32 and beam_src.numel() == shape[0] and beam_src.is_contiguous(), what, "beam_src must be int32 [rows]")
+    _beam_check(0 <= length <= shape[1], what, "length exceeds the cache capacity")
+    table = (C.c_void_p * len(caches))(*[_p(c).value for c in caches])
+    check(_lib.load().evlm_kv_beam_reorder(table, len(caches), shape[0] // num_beams, num_beams, shape[1], shape[2], int(length), _p(beam_src),
+                                           _stream()), what)
+
+
 def rng_bind(state):
     """Bind (or with None unbind) the device uint64 word every dropout site adds to its seed."""
     if state is not None:

@@ -966,6 +966,27 @@ def _kv_cache_of(past_k, past_v, B, nh, E):
     return cache
 
 
+def kv_beam_reorder(past, beam_src, num_beams):
+    """Beam search: re-order a decode loop's `past` IN PLACE (row r takes the row of its item's beam beam_src[r], int32 [rows]) when every
+    layer's K / V are views of a live cache buffer; `past` then stays recognised by _kv_cache_of, so the next step keeps appending in
+    place.  One launch per distinct cache shape (one for an unpruned decoder).  Returns False, touching nothing, when some layer's
+    `past` is not a live cache (KV_CACHE off, or a cache that ran out of spare rows): the caller re-orders by copying."""
+    if not KV_CACHE:
+        return False
+    groups = {}
+    for layer in past:
+        pk, pv = layer[0], layer[1]
+        B, nh, Lp, _ = pk.shape
+        cache = _kv_cache_of(pk, pv, B, nh, nh * 64)
+        if cache is None:
+            return False
+        groups.setdefault((tuple(cache.shape), Lp), []).append(cache)
+    for (_, Lp), caches in groups.items():
+        for i in range(0, len(caches), 32):
+            K.kv_beam_reorder(caches[i:i + 32], beam_src, num_beams, Lp)
+    return True
+
+
 class BertLayerFn(torch.autograd.Function):
     """args: x, key_mask, enc, enc_mask, enc_index, self_head_z, cross_head_z, mlp_z, past_k, past_v, cfg,
              [self: qw,qb,kw,kb,vw,vb,ow,ob,lnw,lnb] [cross: same 10 | omitted] [ffn: w1,b1,w2,b2,lnw,lnb]

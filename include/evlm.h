@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define EVLM_ABI_VERSION 7
+#define EVLM_ABI_VERSION 8
 int evlm_abi_version(void);
 /* Number of kernel launches issued through this library by the calling process (bench gpu_launches). */
 unsigned long long evlm_launch_count(void);
@@ -233,6 +233,34 @@ typedef struct evlm_attn_args {
 int evlm_greedy_select(const float* logits, int64_t ld, int32_t rows, int32_t vocab, const int64_t* unfinished, int64_t pad,
                        const int64_t* eos_host, int32_t n_eos, int64_t* next_token, float* score, int64_t* tokens_to_add,
                        int64_t* unfinished_out, void* stream);
+/* ABI v8 — beam search on the device (transformers 4.12.5's beam_search / BeamSearchScorer / BeamHypotheses, as restated by
+ * eff_bert.py::BertLMHeadModel._beam_search and oracle/beam_search_oracle.py).  rows = batch * beams, 2 <= beams <= 8.
+ * Loop state (device): tokens int64 [rows, width] (history, prompt pre-filled), beam_scores fp32 [rows], beam_src int32 [rows] (source
+ * beam inside the item), done int32 [batch], hyp_tokens int64 [batch, beams, width], hyp_len int32 [batch, beams], hyp_score fp64
+ * [batch, beams], hyp_count int32 [batch], hyp_worst fp64 [batch] (initially 1e9).  Hypothesis scores are fp64, like the host's floats;
+ * cur_len_pow = cur_len ** length_penalty, computed by the caller (the host's own pow), divides every score of the call.
+ * evlm_beam_step: one decode position at history length cur_len (< width) from the step's fp32 logits [rows, ld]: log-softmax,
+ *   repetition penalty on the log-probabilities of every token in the row's history, eos -> -inf while cur_len < min_length, + beam
+ *   score, top 2 * beams over beams x vocab (ties: lowest flat index), BeamSearchScorer.process, BeamHypotheses.add / is_done; the
+ *   history is re-ordered inside the item and the new token written at column cur_len.  Finished items keep their rows (identity
+ *   source, pad token, score 0).  Requires vocab > 2 * beams. */
+int evlm_beam_step(const float* logits, int64_t ld, int32_t batch, int32_t beams, int32_t vocab, int32_t cur_len, int32_t min_length,
+                   float repetition_penalty, double cur_len_pow, int32_t early_stopping, int64_t eos, int64_t pad, int64_t* tokens,
+                   int64_t width, float* beam_scores, int32_t* beam_src, int32_t* done, int64_t* hyp_tokens, int32_t* hyp_len,
+                   double* hyp_score, int32_t* hyp_count, double* hyp_worst, void* stream);
+/* BeamSearchScorer.finalize after the last step (history length cur_len <= width): unfinished items add their live beams; out int64
+ * [batch, max_length] (max_length <= width) = best hypothesis (last of the maximal scores in list order), eos if it is shorter than
+ * max_length, then pad; out_len int32 [batch] = its length. */
+int evlm_beam_finalize(const int64_t* tokens, int64_t width, const float* beam_scores, const int32_t* done, int32_t batch, int32_t beams,
+                       int32_t cur_len, int32_t max_length, double cur_len_pow, int64_t eos, int64_t pad, int64_t* hyp_tokens,
+                       int32_t* hyp_len, double* hyp_score, int32_t* hyp_count, double* hyp_worst, int64_t* out, int32_t* out_len,
+                       void* stream);
+/* In-place re-order of `layers` self-attention KV caches (bf16 [batch * beams, capacity, row_elems], row_elems % 8 == 0, 16-byte
+ * aligned; caches_host: HOST array of device pointers) in one launch: for positions < len, row r takes the row of item(r) * beams +
+ * beam_src[r] (0 <= beam_src < beams).  Positions >= len are untouched. */
+#define EVLM_KV_REORDER_MAX_LAYERS 32
+int evlm_kv_beam_reorder(void* const* caches_host, int32_t layers, int32_t batch, int32_t beams, int64_t capacity, int64_t row_elems,
+                         int32_t len, const int32_t* beam_src, void* stream);
 /* dst[index[i], :] += src[i, :]  (src bf16 [n_src, row_elems], dst fp32 [n_dst, row_elems] pre-zeroed by the caller; fp32 red.add) */
 int evlm_index_add_rows(const void* src_bf16, const int32_t* index, float* dst, int64_t n_src, int64_t row_elems, void* stream);
 /* deterministic variant without atomics on the data: dst_bf16[u, :] = sum_{i: index[i]==u} src_bf16[i, :] (fp32 accumulate);
