@@ -80,7 +80,7 @@ __global__ void __launch_bounds__(256) mse_pairs_fwd_kernel(const evlm_mse_pair*
           if (two) pr.rowdot[r1] = dot1;
         }
       }
-    } else if (vec) {
+    } else if (vec && pr.rowdot == nullptr) {
       int64_t i = tid;
       for (; i + 3 * stride < n4; i += 4 * stride) {
         float4 a[4], b[4];
@@ -105,9 +105,13 @@ __global__ void __launch_bounds__(256) mse_pairs_fwd_kernel(const evlm_mse_pair*
         acc += d * d;
       }
     } else {
+      // unaligned maps (or rows the warp-per-row loop cannot take) that want the row sums leave them one atomic per element, as the
+      // backward's scalar path does
       for (int64_t j = tid; j < pr.n; j += stride) {
-        const float d = ld1_any(pr.s, pr.s_dtype, j) - ld1_any(pr.t, pr.t_dtype, j);
+        const float a = ld1_any(pr.s, pr.s_dtype, j);
+        const float d = a - ld1_any(pr.t, pr.t_dtype, j);
         acc += d * d;
+        if (pr.rowdot != nullptr) atomicAdd(pr.rowdot + j / pr.row_len, d * a);
       }
     }
     acc = block_sum(acc, red);

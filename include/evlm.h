@@ -281,7 +281,8 @@ typedef struct evlm_mse_pair {
   int64_t n; float scale; int32_t s_dtype; int32_t t_dtype; int32_t pad;
   /* ABI v6, backward only: when rowdot != NULL the pair is an attention map with rows of row_len elements (row_len % 4 == 0, n %
    * row_len == 0) and rowdot[r] += sum_j ds[r, j] * s[r, j] — the "sum_j dP_ij P_ij" term of the softmax backward, produced here
-   * from values that are in registers anyway instead of by a pre-kernel that re-reads both maps (evlm_attn_args.dp_rowdot).        */
+   * from values that are in registers anyway instead of by a pre-kernel that re-reads both maps (evlm_attn_args.dp_rowdot).
+   * The forward leaves rowdot[r] = sum_j (s - t)[r, j] * s[r, j] (unscaled) on every path; rowdot must arrive zeroed.            */
   float* rowdot; int64_t row_len;
 } evlm_mse_pair;
 int evlm_mse_pairs_fwd(const evlm_mse_pair* pairs_dev, int npairs, float* out /*[npairs], zeroed by callee*/, void* stream);
