@@ -32,6 +32,7 @@ def _default_tokenizer(path):
 class XVLMForCaptioning(XVLMBase):
     """models/model_generation.py:61-218 — un-gated captioning model (the distillation teacher of Eff_Captioning.py)."""
     gated = False
+    gates_folded = False        # set by prune.materialize: the deterministic gates live in the (physically pruned) weights
 
     def __init__(self, config, tokenizer=None):
         super().__init__(config, load_vision_params=False, load_text_params=False, use_contrastive_loss=False, use_matching_loss=False,
@@ -60,7 +61,7 @@ class XVLMForCaptioning(XVLMBase):
         return self.tokenizer(caption, padding="longest", truncation=True, max_length=self.max_tokens, return_tensors="pt").to(device)
 
     def _zs(self, training):
-        if not self.gated:
+        if not self.gated or self.gates_folded:
             return None
         if training:
             return self.l0_module.forward(training=True)
@@ -68,6 +69,9 @@ class XVLMForCaptioning(XVLMBase):
             return self.l0_module.forward(training=False)
 
     def forward(self, image, caption, output_attentions=None, output_hidden_states=None):
+        if self.gates_folded:
+            raise RuntimeError("this captioning model was materialised (prune.materialize): its gates are folded into pruned weights, so the "
+                               "training forward, which applies freshly sampled full-width gates, cannot run on it; use generate()")
         zs = self._zs(True)                                                    # model_generation.py:350 (sampled even when unused)
         dec_head = dec_mlp = vis_head = vis_mlp = None
         if zs is not None:
@@ -100,7 +104,9 @@ class XVLMForCaptioning(XVLMBase):
         """model_generation.py:407-484.  greedy / sample: the reference's own decode loop (`_generate_no_beam_search`); otherwise beam
         search (`BertLMHeadModel.generate`: transformers 4.12.5's algorithm restated, parity unpinned; on CUDA the scorer runs on the device).
         return_ids=True (extension) also returns the generated token ids; sync_free=True (extension) decodes to max_length without
-        host checks or reads (same result, graph-capturable; beam-search ids are then [batch, max_length], pad-filled; see eff_bert)."""
+        host checks or reads (same result, graph-capturable; beam-search ids are then [batch, max_length], pad-filled; see eff_bert).
+        After prune.materialize the model decodes WITHOUT gates, on the vision tower and on the decoder, in every mode: the decoder's
+        beam-search gates are folded into its weights, and greedy / sampling then run that folded decoder."""
         zs = self._zs(False)
         vis_head = vis_mlp = None
         if zs is not None:

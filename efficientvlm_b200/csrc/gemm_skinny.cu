@@ -34,6 +34,15 @@ __device__ __forceinline__ void mma_bf16_16816(float (&c)[4], uint32_t a0, uint3
                : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
+// The first r (1..7) bf16 elements of an 8-element group, the rest zero.
+__device__ __forceinline__ uint4 keep_first_elems(uint4 v, const int r) {
+  const uint32_t m0 = r >= 2 ? 0xffffffffu : 0x0000ffffu;
+  const uint32_t m1 = r >= 4 ? 0xffffffffu : r == 3 ? 0x0000ffffu : 0u;
+  const uint32_t m2 = r >= 6 ? 0xffffffffu : r == 5 ? 0x0000ffffu : 0u;
+  const uint32_t m3 = r == 7 ? 0x0000ffffu : 0u;
+  return make_uint4(v.x & m0, v.y & m1, v.z & m2, v.w & m3);
+}
+
 template <int MB>
 __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const evlm_gemm_args g, const int ks, const int chunks_per_slice) {
   namespace cg = cooperative_groups;
@@ -69,13 +78,15 @@ __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const evlm_gemm
     brow[nb] = n < g.N ? B + (int64_t)n * g.ldb : nullptr;
   }
   const uint4 zero4 = make_uint4(0u, 0u, 0u, 0u);
+  // The main loop takes the whole 8-element groups [0, K8); a partial last group (K % 8 != 0) is added after it, masked in registers.
+  const int K8 = g.K & ~7;
   for (int c0 = c_begin + khalf; c0 < c_end; c0 += 2 * SK_UNROLL) {
     uint4 av[SK_UNROLL][MB][2], bv[SK_UNROLL][2];
 #pragma unroll
     for (int u = 0; u < SK_UNROLL; ++u) {
       const int c = c0 + 2 * u;
-      const int k = c * 32 + t * 8;      // K % 8 == 0: a lane's 8 elements are all valid or all beyond K
-      const bool kok = c < c_end && k < g.K;
+      const int k = c * 32 + t * 8;      // a lane's 8 elements are all below K8 or all at / beyond it
+      const bool kok = c < c_end && k < K8;
 #pragma unroll
       for (int nb = 0; nb < 2; ++nb) bv[u][nb] = (kok && brow[nb]) ? __ldg(reinterpret_cast<const uint4*>(brow[nb] + k)) : zero4;
 #pragma unroll
@@ -93,6 +104,31 @@ __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const evlm_gemm
           mma_bf16_16816(acc[mb][nb], av[u][mb][0].x, av[u][mb][1].x, av[u][mb][0].y, av[u][mb][1].y, bv[u][nb].x, bv[u][nb].y);
           mma_bf16_16816(acc[mb][nb], av[u][mb][0].z, av[u][mb][1].z, av[u][mb][0].w, av[u][mb][1].w, bv[u][nb].z, bv[u][nb].w);
         }
+  }
+  // Partial last group [K8, K): it sits in chunk ct at lane column tt, which belongs to this slice's warps of one k half.  The 16-byte
+  // load stays inside the row's pitch (16-byte aligned base and pitch, checked by gemm_skinny_try); the elements at K and beyond are
+  // zeroed in registers on both operands, so whatever the pitch padding holds (NaN included) never reaches the product.
+  if (K8 != g.K) {
+    const int ct = K8 >> 5, tt = (K8 & 31) >> 3, r = g.K - K8;
+    if (ct >= c_begin && ct < c_end && ((ct - c_begin) & 1) == khalf) {
+      const bool mine = t == tt;
+      uint4 at[MB][2], bt[2];
+#pragma unroll
+      for (int nb = 0; nb < 2; ++nb)
+        bt[nb] = (mine && brow[nb]) ? keep_first_elems(__ldg(reinterpret_cast<const uint4*>(brow[nb] + K8)), r) : zero4;
+#pragma unroll
+      for (int mb = 0; mb < MB; ++mb)
+#pragma unroll
+        for (int h = 0; h < 2; ++h)
+          at[mb][h] = (mine && arow[mb][h]) ? keep_first_elems(__ldg(reinterpret_cast<const uint4*>(arow[mb][h] + K8)), r) : zero4;
+#pragma unroll
+      for (int mb = 0; mb < MB; ++mb)
+#pragma unroll
+        for (int nb = 0; nb < 2; ++nb) {
+          mma_bf16_16816(acc[mb][nb], at[mb][0].x, at[mb][1].x, at[mb][0].y, at[mb][1].y, bt[nb].x, bt[nb].y);
+          mma_bf16_16816(acc[mb][nb], at[mb][0].z, at[mb][1].z, at[mb][0].w, at[mb][1].w, bt[nb].z, bt[nb].w);
+        }
+    }
   }
   // partial sums -> shared memory (accumulator fragment: c0,c1 = (row g, cols 2t, 2t+1); c2,c3 = (row g+8, same cols))
 #pragma unroll
@@ -145,11 +181,14 @@ __global__ void __launch_bounds__(SK_THREADS) gemm_skinny_kernel(const evlm_gemm
 }
 
 // Returns -1 when the product is not a small-M forward one (the caller then runs the tcgen05 kernel), else the launch status.
+// Any K >= 1 is taken; the kernel's 16-byte operand loads need 16-byte aligned bases and row pitches of A and B (ops.alloc16 and the
+// weight shadows provide them), a partial last 8-element group is masked in registers.
 int gemm_skinny_try(const evlm_gemm_args* a, void* stream) {
   static const bool off = getenv("EVLM_GEMM_NO_SKINNY") != nullptr;   // profiling knob: every product on the tcgen05 kernel
   if (off || a->M > 32 || a->a_mn || a->b_mn || a->epi_mode != EVLM_EPI_FORWARD || a->splits > 1 || a->accumulate ||
-      a->dropout_p > 0.f || a->m_limit || a->n_limit || a->k_limit || (a->K & 7))
+      a->dropout_p > 0.f || a->m_limit || a->n_limit || a->k_limit || a->K < 1)
     return -1;
+  if ((reinterpret_cast<uintptr_t>(a->A) & 15) || (reinterpret_cast<uintptr_t>(a->B) & 15) || (a->lda & 7) || (a->ldb & 7)) return -1;
   const int col_blocks = (a->N + 63) / 64, nchunks = (a->K + 31) / 32;
   int ks = 1;                                    // k slices per column block: about two CTAs per SM, at least 4 chunks per slice
   while (ks < 8 && col_blocks * ks < 2 * 148 && nchunks / (ks * 2) >= 4) ks *= 2;

@@ -227,6 +227,16 @@ class BertLayer(nn.Module):
         return outputs + (present,)
 
 
+def layer_gate_rows(i, fusion_layer):
+    """(self-attention head row, cross-attention head row or None, FFN row) of the gate tensors that BertEncoder.forward hands layer i.
+    Quirk Q1 (eff_bert.py:612-620): head gates of fusion layers come in (self, cross) pairs, and in multi_modal mode with concatenated
+    gates the fusion layers re-use the *text* slots.  prune.py folds a captioning decoder's gates through the same table."""
+    if i >= fusion_layer:
+        first = (i - fusion_layer) * 2
+        return first, first + 1, i - fusion_layer
+    return i, None, i
+
+
 class BertEncoder(nn.Module):
     def __init__(self, config):
         super().__init__()
@@ -256,15 +266,10 @@ class BertEncoder(nn.Module):
             layer_module = self.layer[i]
             if output_hidden_states:
                 all_hidden_states = all_hidden_states + (hidden_states,)
-            # gate indexing incl. quirk Q1 (eff_bert.py:612-620): head gates of fusion layers come in (self, cross) pairs,
-            # and in multi_modal mode with concatenated gates the fusion layers re-use the *text* slots.
-            if i >= self.fusion_layer and head_z is not None:
-                first = (i - self.fusion_layer) * 2
-                cur_head_z = (head_z[first], head_z[first + 1])
-                cur_mlp_z = mlp_z[i - self.fusion_layer]
-            elif head_z is not None:
-                cur_head_z = head_z[i]
-                cur_mlp_z = mlp_z[i]
+            if head_z is not None:
+                self_row, cross_row, mlp_row = layer_gate_rows(i, self.fusion_layer)
+                cur_head_z = head_z[self_row] if cross_row is None else (head_z[self_row], head_z[cross_row])
+                cur_mlp_z = mlp_z[mlp_row]
             else:
                 cur_mlp_z, cur_head_z = None, None
             past_key_value = past_key_values[i] if past_key_values is not None else None

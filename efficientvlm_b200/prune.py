@@ -7,14 +7,22 @@ models), `utils/vqa_utils.py:37-293` and `utils/caption_utils.py` (models with a
   2. `prune_model_with_z`: `prune_heads` every head whose gate is exactly 0 and slice away the FFN columns whose gate is 0.
 The layer counts come from the gate tensors instead of the literals 6 / 3 / 3 / 3 of the reference files.
 
-The pruned modules run on the same kernels (tests/test_host_logic.py::test_materialised_vqa_model_matches_gated_networks): the
-GEMMs accept any N / K that is a multiple of 8 elements after padding the bf16 shadow pitch, attention takes `num_heads` from the
-module.  Like the reference, a layer whose heads or FFN columns are ALL pruned is not representable by the forward code
-(the reference sets the Linear to None and then fails in forward); this module refuses to produce such a layer.
+The pruned modules run on the same kernels: the GEMMs take any N / K (the bf16 operands keep 16-byte row pitches, and the small-M
+weight-stream kernel of the decode steps masks a partial last 8-element group of K), attention takes `num_heads` from the module.
+Like the reference, a layer whose heads or FFN columns are ALL pruned is not representable by the forward code (the reference sets
+the Linear to None and then fails in forward); this module refuses to produce such a layer.
+
+Captioning models (`text_encoder is None`, the XVLML0Module gates drive `text_decoder`): the decoder's gates are folded exactly as the
+gated decoder applies them on the one decode path where the reference gates it, beam search (captioning.XVLMForCaptioning.generate):
+head_z = cat(text_head_z, cross_head_z) and mlp_z = cat(text_intermediate_z, cross_intermediate_z), indexed per layer by
+`eff_bert.layer_gate_rows` (quirk Q1: with fusion layer F, layer i >= F takes self row 2(i - F), cross row 2(i - F) + 1 and FFN row
+i - F, so the trailing cross_* rows are never read).  The reference's utils/caption_utils.py is not available, so parity with its
+captioning recipe is unpinned; the target is the gated model's own decode (tests/test_caption_materialize.py).
 """
 import torch
 
 from . import ops
+from .eff_bert import layer_gate_rows
 from .eff_vit import prune_linear_layer
 
 DIMS_PER_HEAD = 64
@@ -38,12 +46,44 @@ def _scale_value(att_self, head_z):
     att_self.value.bias.data = att_self.value.bias.data.mul(hz)
 
 
+def caption_decoder_gates(zs, decoder):
+    """Per decoder layer: (self head gate row, cross head gate row or None, FFN gate row), the rows the gated decoder of a captioning
+    model applies to that layer (see the module docstring)."""
+    heads = _rows(torch.cat((zs["text_head_z"], zs["cross_head_z"]), dim=0))
+    mlps = _rows(torch.cat((zs["text_intermediate_z"], zs["cross_intermediate_z"]), dim=0))
+    out = []
+    for i in range(len(decoder.encoder.layer)):
+        s, c, m = layer_gate_rows(i, decoder.encoder.fusion_layer)
+        out.append((heads[s], None if c is None else heads[c], mlps[m]))
+    return out
+
+
+def _caption_plan(gates):
+    """Per decoder layer: (self heads to prune, cross heads to prune or None, FFN columns to keep); refuses a layer left empty."""
+    return [(_zero_heads(s, "decoder self", i), None if c is None else _zero_heads(c, "decoder cross", i), _kept_columns(m, "decoder", i))
+            for i, (s, c, m) in enumerate(gates)]
+
+
+def _is_captioner(model, zs):
+    return _bert_of(model, "text_encoder") is None and _bert_of(model, "text_decoder") is not None and "text_head_z" in zs
+
+
 @torch.no_grad()
 def update_params(model, zs):
     """vqa_utils.py:37-104 / xvlm_utils.py:37-85: gate values folded into value projections and FFN down-projections."""
     vision = model.vision_encoder
     text = _bert_of(model, "text_encoder")
     decoder = _bert_of(model, "text_decoder")
+    if _is_captioner(model, zs):
+        gates = caption_decoder_gates(zs, decoder)
+        _caption_plan(gates)                  # a layer that would be left empty is refused before any weight changes
+        for blk, (self_z, cross_z, mlp_z) in zip(decoder.encoder.layer, gates):
+            _scale_value(blk.attention.self, self_z)
+            if cross_z is not None:
+                _scale_value(blk.crossattention.self, cross_z)
+            d = blk.output.dense
+            d.weight.data = d.weight.data.mul(mlp_z.to(d.weight.device))
+        zs = {k: v for k, v in zs.items() if k.startswith("vision_")}
     n_text = zs["text_head_z"].shape[0] if "text_head_z" in zs else (zs["text_intermediate_z"].shape[0] if "text_intermediate_z" in zs else 0)
     if "vision_intermediate_z" in zs:
         for layer, z in enumerate(_rows(zs["vision_intermediate_z"])):
@@ -85,25 +125,27 @@ def update_params(model, zs):
     ops.invalidate_weight_cache()
 
 
+def _zero_heads(row, what, layer):
+    idx = torch.where(row == 0)[0].tolist()
+    if len(idx) == row.numel():
+        raise NotImplementedError("%s layer %d: every head is pruned; the forward code (reference and B200) cannot run a layer "
+                                  "without heads" % (what, layer))
+    return idx
+
+
+def _kept_columns(row, what, layer):
+    keep = row.nonzero().reshape(-1).tolist()
+    if not keep:
+        raise NotImplementedError("%s layer %d: every FFN column is pruned; the forward code cannot run a layer without an FFN" % (what, layer))
+    return keep
+
+
 def _heads_to_prune(z, what):
-    out = {}
-    for layer, row in enumerate(_rows(z)):
-        idx = torch.where(row == 0)[0].tolist()
-        if len(idx) == row.numel():
-            raise NotImplementedError("%s layer %d: every head is pruned; the forward code (reference and B200) cannot run a layer "
-                                      "without heads" % (what, layer))
-        out[layer] = idx
-    return out
+    return {layer: _zero_heads(row, what, layer) for layer, row in enumerate(_rows(z))}
 
 
 def _kept_dims(z, what):
-    out = {}
-    for layer, row in enumerate(_rows(z)):
-        keep = row.nonzero().reshape(-1).tolist()
-        if not keep:
-            raise NotImplementedError("%s layer %d: every FFN column is pruned; the forward code cannot run a layer without an FFN" % (what, layer))
-        out[layer] = keep
-    return out
+    return {layer: _kept_columns(row, what, layer) for layer, row in enumerate(_rows(z))}
 
 
 def prune_intermediate_layers(bert, keep_dims, device=None):
@@ -132,6 +174,14 @@ def prune_model_with_z(zs, model):
     vision = model.vision_encoder
     text = _bert_of(model, "text_encoder")
     decoder = _bert_of(model, "text_decoder")
+    if _is_captioner(model, zs):
+        plan = _caption_plan(caption_decoder_gates(zs, decoder))
+        for blk, (self_heads, cross_heads, _) in zip(decoder.encoder.layer, plan):
+            blk.attention.prune_heads(self_heads)
+            if cross_heads is not None:
+                blk.crossattention.prune_heads(cross_heads)
+        prune_intermediate_layers(decoder, {i: keep for i, (_, _, keep) in enumerate(plan)})
+        zs = {k: v for k, v in zs.items() if k.startswith("vision_")}
     if "vision_head_z" in zs:
         vision.prune_heads(_heads_to_prune(zs["vision_head_z"], "vision"))
     if "text_head_z" in zs:
@@ -154,10 +204,12 @@ def prune_model_with_z(zs, model):
 def materialize(model, zs=None):
     """update_params + prune_model_with_z with the model's own deterministic masks (l0_module.forward(training=False)) by
     default.  Returns the per-module sizes `l0_module.calculate_model_size` reports.  The pruned model is then run WITHOUT gates
-    (the reference's `fake_forward`, model_generation.py:214-230): see `efficientvlm_b200.vqa.XVLMForVQA.forward(..., use_gates=False)`."""
+    (the reference's `fake_forward`, model_generation.py:214-230): see `efficientvlm_b200.vqa.XVLMForVQA.forward(..., use_gates=False)`.
+    Sets `model.gates_folded`: a captioning model's `generate` then runs without gates, and its `forward` refuses to run."""
     if zs is None:
         with torch.no_grad():
             zs = model.l0_module.forward(training=False)
     update_params(model, zs)
     prune_model_with_z(zs, model)
+    model.gates_folded = True
     return model.l0_module.calculate_model_size(zs) if hasattr(model, "l0_module") else None
