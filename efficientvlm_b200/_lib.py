@@ -75,6 +75,8 @@ PROTOTYPES = {
     "evlm_launch_count": (C.c_ulonglong, []),
     "evlm_reset_launch_count": (None, []),
     "evlm_gemm_bf16": (c_i32, [C.POINTER(GemmArgs), c_p]),
+    "evlm_gemm_fp8": (c_i32, [C.POINTER(GemmArgs), c_p, c_p, c_p]),
+    "evlm_quant_rows_e4m3": (c_i32, [c_p, c_i32, c_i64, c_i64, c_i64, c_p, c_i64, c_p, c_p]),
     "evlm_sgemm": (c_i32, [c_i32, c_i32, c_i32, c_f, c_p, c_i64, c_i32, c_p, c_i64, c_i32, c_f, c_p, c_i64, c_p, c_i32, c_p]),
     "evlm_dot": (c_i32, [c_p, c_p, c_i64, c_f, c_p, c_i32, c_p]),
     "evlm_cast_f32_to_bf16": (c_i32, [c_p, c_i64, c_p, c_i64, c_i64, c_i64, c_f, c_u64, c_u32, c_p]),
@@ -137,7 +139,7 @@ PROTOTYPES = {
     "evlm_kv_beam_reorder": (c_i32, [C.POINTER(c_p), c_i32, c_i32, c_i32, c_i64, c_i64, c_i32, c_p, c_p]),
 }
 
-ABI_VERSION = 8   # must equal EVLM_ABI_VERSION in include/evlm.h
+ABI_VERSION = 9   # must equal EVLM_ABI_VERSION in include/evlm.h
 _lib = None
 
 

@@ -36,6 +36,20 @@ static inline int make_tmap_bf16(CUtensorMap* tm, const void* base, int64_t rows
   return r == CUDA_SUCCESS ? 0 : EVLM_EINVAL;
 }
 
+// 2-D e4m3 tensor map (UINT8: the TMA unit only moves bytes) over a row-major [rows, cols] matrix with a row pitch of ld bytes;
+// box = {128 cols (128 B, SWIZZLE_128B), box_rows} — the byte geometry of the bf16 map above.  Columns >= cols are filled with 0.
+static inline int make_tmap_e4m3(CUtensorMap* tm, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
+  auto fn = get_encode_fn();
+  if (!fn) return (int)cudaErrorNotSupported;
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)ld};
+  cuuint32_t box[2] = {128u, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1u, 1u};
+  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return r == CUDA_SUCCESS ? 0 : EVLM_EINVAL;
+}
+
 // Tensor map for EPILOGUE STORES of a row-major [rows, cols] matrix (bf16 or fp32): box = {16 cols, 32 rows}, i.e. one
 // epilogue warp's chunk; the 32-byte (bf16) / 64-byte (fp32) box rows are swizzled so that a thread writing its own row and
 // the TMA engine reading the box are both bank-conflict free.  Needs a 16-byte aligned base and row pitch.

@@ -29,11 +29,15 @@
 namespace evlm {
 
 std::atomic<unsigned long long> g_launch_count{0};
-int gemm_skinny_try(const evlm_gemm_args* a, void* stream);   // gemm_skinny.cu: M <= 32 forward products (decode steps)
+// gemm_skinny.cu: M <= 32 forward products (decode steps); a_scale != nullptr: e4m3 operands
+int gemm_skinny_try(const evlm_gemm_args* a, const float* a_scale, const float* b_scale, void* stream);
 
 constexpr int BLOCK_M = 128;
-constexpr int BLOCK_K = 64;
+constexpr int BLOCK_K = 64;                 // bf16: 64 elements = 128-byte rows (one SWIZZLE_128B atom)
 constexpr int UMMA_K = 16;
+// F8 (evlm_gemm_fp8, e4m3 operands): the same 128-byte rows hold 128 elements; a stage is four kind::f8f6f4 MMAs of K = 32, the
+// descriptor advancing 32 B per step exactly as for bf16, so stage bytes, swizzle and descriptors are shared.
+constexpr int BLOCK_K_F8 = 128;
 constexpr int NUM_EPI_WARPS = 16;  // 16 warps: the epilogue is latency-bound per warp, thread-level parallelism hides it
 constexpr int NUM_EPI_THREADS = NUM_EPI_WARPS * 32;
 constexpr int NUM_THREADS = 64 + NUM_EPI_THREADS;
@@ -66,6 +70,8 @@ struct GemmParams {
   int side_kind;          // DB epilogue: 0 none, 1 fp32 box (2 KB), 2 bf16 box (1 KB)
   evlm_gemm_args g;
   int m_tiles, n_tiles, k_blocks, splits, kb_per_split;
+  const float* a_scale;   // F8: [M] row scales of A
+  const float* b_scale;   // F8: [N] row scales of B (output channels)
 };
 
 // value and derivative of the activation (fast formulations, see evlm_common.cuh)
@@ -317,8 +323,27 @@ __device__ __forceinline__ void tmem_load_chunk(uint32_t taddr, float (&v)[CH], 
   for (int j = 0; j < CH; ++j) v[j] = __uint_as_float(r[j]);
 }
 
+// F8: the accumulator of e4m3 products times a_scale[row] * b_scale[col], before anything else of the epilogue
+template <bool F8>
+__device__ __forceinline__ void apply_f8_scales(const GemmParams& p, int row, const ChunkGeom& cg, float (&v)[CH]) {
+  if constexpr (F8) {
+    const float sa = row < p.g.M ? __ldg(p.a_scale + row) : 0.f;
+    const float* sp = p.b_scale + cg.col0;
+    if (cg.ncols == CH) {   // (col0 is a multiple of 16 and the scale vector is allocated 16-byte aligned)
+#pragma unroll
+      for (int j = 0; j < CH; j += 4) {
+        const float4 q = __ldg(reinterpret_cast<const float4*>(sp + j));
+        v[j] *= sa * q.x; v[j + 1] *= sa * q.y; v[j + 2] *= sa * q.z; v[j + 3] *= sa * q.w;
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < CH; ++j) v[j] *= sa * (j < cg.ncols ? sp[j] : 0.f);
+    }
+  }
+}
+
 // One 32-row x CH-column chunk through the epilogue; `row` is this thread's row, `cg` the chunk as a whole.
-template <int EPI>
+template <int EPI, bool F8>
 __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, uint32_t taddr, float* st, const float* bias_s, const float* gate_s,
                                                int lane, int row, const ChunkGeom& cg, int split, bool add, float keep_scale, bool acc_zero) {
   const evlm_gemm_args& g = p.g;
@@ -344,6 +369,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, uint32_t tad
     if constexpr (EPI == EPI_LINEAR) {
       // plain GEMMs: no column stage (its two barriers per tile cost more than the bias load they would hide)
       tmem_load_chunk(taddr, v, acc_zero);
+      apply_f8_scales<F8>(p, row, cg, v);
       if (g.bias != nullptr && split == 0) {
         float b[CH];
         load_cols_f32(g.bias + col0, b, ncols);
@@ -352,6 +378,7 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, uint32_t tad
       }
     } else {
       tmem_load_chunk(taddr, v, acc_zero);
+      apply_f8_scales<F8>(p, row, cg, v);
       float b[CH];   // zeros when there is no bias
       load_cols_smem(bias_s, b);
 #pragma unroll
@@ -473,7 +500,7 @@ __device__ __forceinline__ void box_put_row_bf16(uint8_t* base, int lane, const 
 // One chunk.  `buf` holds this chunk's side operand (when has_side) and receives its outputs; `nbuf` is the other buffer: the
 // previous chunk's stores are drained from it and the NEXT chunk's side operand is requested into it before anything else happens,
 // so that load has this whole chunk to land.
-template <int EPI>
+template <int EPI, bool F8>
 __device__ __forceinline__ void epilogue_chunk_db(const GemmParams& p, uint32_t taddr, uint8_t* buf, uint8_t* nbuf, const float* bias_s,
                                                   const float* gate_s, int lane, int row, const ChunkGeom& cg, int split, bool add,
                                                   float keep_scale, bool has_side, uint32_t side_bar, uint32_t side_phase, uint32_t next_bar,
@@ -504,6 +531,7 @@ __device__ __forceinline__ void epilogue_chunk_db(const GemmParams& p, uint32_t 
       else box_get_row_bf16(buf, lane, q);
     }
     tmem_load_chunk(taddr, v, acc_zero);
+    apply_f8_scales<F8>(p, row, cg, v);
     if constexpr (EPI == EPI_LINEAR) {
       if (g.bias != nullptr && split == 0) {
         float b[CH];
@@ -591,9 +619,10 @@ __device__ __forceinline__ void epilogue_chunk_db(const GemmParams& p, uint32_t 
   }
 }
 
-template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool DB>
+template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool DB, bool F8>
 __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __grid_constant__ GemmParams p) {
   using Cfg = GemmCfg<BLOCK_N, DB>;
+  constexpr int BK = F8 ? BLOCK_K_F8 : BLOCK_K;   // elements per k block (128 bytes per operand row either way)
   extern __shared__ __align__(1024) uint8_t smem_raw[];   // SWIZZLE_128B operand tiles need 1024-byte alignment
   const uint32_t smem_base = smem_u32(smem_raw);
   if ((smem_base & 1023u) != 0) __trap();
@@ -646,7 +675,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
   if (g.m_limit) m_tiles_e = min(m_tiles_e, (max(0, __ldg(g.m_limit)) + BLOCK_M - 1) / BLOCK_M);
   if (g.n_limit) n_tiles_e = min(n_tiles_e, (max(0, __ldg(g.n_limit)) + BLOCK_N - 1) / BLOCK_N);
   if (g.k_limit) {
-    k_blocks_e = min(k_blocks_e, (max(0, __ldg(g.k_limit)) + BLOCK_K - 1) / BLOCK_K);
+    k_blocks_e = min(k_blocks_e, (max(0, __ldg(g.k_limit)) + BK - 1) / BK);
     kbps_e = (k_blocks_e + p.splits - 1) / p.splits;
   }
   const int total_work = m_tiles_e * n_tiles_e * p.splits;
@@ -671,7 +700,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
           const uint32_t sa = smem_base + s * Cfg::kStageBytes;
           const uint32_t sb = sa + Cfg::kABytes;
           mbar_expect_tx(full_bar(s), Cfg::kStageBytes);
-          const int k0 = kb * BLOCK_K;
+          const int k0 = kb * BK;
           if (!A_MN) {
             tma_load_2d(sa, &p.tma_a, k0, m0, full_bar(s));
           } else {
@@ -692,7 +721,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
     // ===================== MMA issuer =====================
     if (lane == 0) {
       // instruction descriptor: D=f32, A=B=bf16, majors, N>>3, M>>4
-      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((A_MN ? 1u : 0u) << 15) | ((B_MN ? 1u : 0u) << 16) |
+      // (F8, kind::f8f6f4: bits 7-9 / 10-12 = A / B format, E4M3 = 0; the other fields are laid out as for kind::f16)
+      const uint32_t idesc = (1u << 4) | (F8 ? 0u : (1u << 7) | (1u << 10)) | ((A_MN ? 1u : 0u) << 15) | ((B_MN ? 1u : 0u) << 16) |
                              ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)(BLOCK_M >> 4) << 24);
       int s = 0;
       uint32_t ph = 0;
@@ -714,7 +744,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
           for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
             const uint64_t adesc = A_MN ? make_desc_mnmajor(sa + k * 2048) : make_desc_kmajor(sa + k * 32);
             const uint64_t bdesc = B_MN ? make_desc_mnmajor(sb + k * 2048) : make_desc_kmajor(sb + k * 32);
-            umma_bf16(tmem_d, adesc, bdesc, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
+            if constexpr (F8) umma_e4m3(tmem_d, adesc, bdesc, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
+            else umma_bf16(tmem_d, adesc, bdesc, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
           }
           umma_commit(empty_bar(s));  // frees the smem stage once these MMAs have read it
           if (++s == Cfg::kStages) { s = 0; ph ^= 1; }
@@ -816,14 +847,14 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
             int nw = w, nci = (c - part * CPP) / CH, nsplit = 0;
             const bool has_next = next_chunk(nw, nci, ng, nsplit);
             const bool hs = side_wanted(split);
-            epilogue_chunk_db<EPI>(p, tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * BLOCK_N + c), dbuf + cb * 2048,
+            epilogue_chunk_db<EPI, F8>(p, tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * BLOCK_N + c), dbuf + cb * 2048,
                                    dbuf + (cb ^ 1) * 2048, cv + (c - part * CPP), cv + CPP + (c - part * CPP), lane, cg.row0 + lane, cg, split,
                                    add, keep_scale, hs, side_bar + 8u * cb, side_uses[cb] & 1u, side_bar + 8u * (cb ^ 1),
                                    has_next && side_wanted(nsplit), ng.col0, ng.row0, acc_zero);
             if (hs) ++side_uses[cb];
             cb ^= 1;
           } else {
-            epilogue_chunk<EPI>(p, tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * BLOCK_N + c), st, cv + (c - part * CPP),
+            epilogue_chunk<EPI, F8>(p, tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(as * BLOCK_N + c), st, cv + (c - part * CPP),
                                 cv + CPP + (c - part * CPP), lane, cg.row0 + lane, cg, split, add, keep_scale, acc_zero);
           }
         }
@@ -846,11 +877,11 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tcgen05_kernel(const __gr
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool DB = false>
+template <int BLOCK_N, bool A_MN, bool B_MN, int EPI, bool DB = false, bool F8 = false>
 static int launch(const GemmParams& p, int grid, cudaStream_t st) {
   using Cfg = GemmCfg<BLOCK_N, DB>;
   static_assert(Cfg::kSmemBytes <= 232448, "shared memory budget");
-  auto kern = gemm_tcgen05_kernel<BLOCK_N, A_MN, B_MN, EPI, DB>;
+  auto kern = gemm_tcgen05_kernel<BLOCK_N, A_MN, B_MN, EPI, DB, F8>;
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(once, [&] { attr_err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes); });
@@ -877,6 +908,16 @@ static int dispatch(const GemmParams& p, int grid, cudaStream_t st, int a_mn, in
   if (a_mn && b_mn) return launch<BLOCK_N, true, true, EPI_LINEAR>(p, grid, st);
   return launch<BLOCK_N, true, false, EPI_LINEAR>(p, grid, st);
 }
+// F8: the forward configurations inference reaches (the double-buffered epilogue serves the K <= 1024 residual projections)
+template <int BLOCK_N>
+static int dispatch_f8(const GemmParams& p, int grid, cudaStream_t st, int epi, bool db) {
+  if (epi == EPI_LINEAR)
+    return db ? launch<BLOCK_N, false, false, EPI_LINEAR, true, true>(p, grid, st) : launch<BLOCK_N, false, false, EPI_LINEAR, false, true>(p, grid, st);
+  if (epi == EPI_ACT_FWD && !db) return launch<BLOCK_N, false, false, EPI_ACT_FWD, false, true>(p, grid, st);
+  return EVLM_EUNSUPPORTED;
+}
+
+static int gemm_tcgen05_run(const evlm_gemm_args* a, const float* a_scale, const float* b_scale, void* stream);
 
 }  // namespace evlm
 
@@ -901,9 +942,38 @@ extern "C" int evlm_gemm_bf16(const evlm_gemm_args* a, void* stream) {
   if (a->dropout_p < 0.f || a->dropout_p >= 1.f) return EVLM_EINVAL;
   if (a->epi_mode == EVLM_EPI_FORWARD && a->act == EVLM_ACT_NONE && a->gate_mode == EVLM_GATE_NONE && a->aux_out) return EVLM_EINVAL;
   {
-    const int rc_skinny = gemm_skinny_try(a, stream);
+    const int rc_skinny = gemm_skinny_try(a, nullptr, nullptr, stream);
     if (rc_skinny != -1) return rc_skinny;
   }
+  return gemm_tcgen05_run(a, nullptr, nullptr, stream);
+}
+
+extern "C" int evlm_gemm_fp8(const evlm_gemm_args* a, const float* a_scale, const float* b_scale, void* stream) {
+  using namespace evlm;
+  if (!a || !a->A || !a->B || !a->D || !a_scale || !b_scale) return EVLM_EINVAL;
+  if (a->M <= 0 || a->N <= 0 || a->K <= 0) return EVLM_EINVAL;
+  // TMA and the weight-stream kernel's 16-byte lane loads: 16-byte aligned bases and row pitches (e4m3: pitch in bytes)
+  if ((reinterpret_cast<uintptr_t>(a->A) & 15) || (reinterpret_cast<uintptr_t>(a->B) & 15) || (a->lda % 16) || (a->ldb % 16)) return EVLM_EINVAL;
+  if (a->lda < a->K || a->ldb < a->K) return EVLM_EINVAL;
+  if (a->a_mn || a->b_mn) return EVLM_EINVAL;
+  if (a->d_dtype != EVLM_BF16 && a->d_dtype != EVLM_F32) return EVLM_EINVAL;
+  if (a->epi_mode != EVLM_EPI_FORWARD || a->dropout_p != 0.f || a->splits > 1 || a->accumulate || a->gate_mode != EVLM_GATE_NONE || a->gate)
+    return EVLM_EINVAL;
+  if (a->m_limit || a->n_limit || a->k_limit) return EVLM_EINVAL;
+  if (a->act != EVLM_ACT_NONE && a->act != EVLM_ACT_QUICK_GELU && a->act != EVLM_ACT_GELU_ERF) return EVLM_EINVAL;
+  if (a->act == EVLM_ACT_NONE && a->aux_out) return EVLM_EINVAL;
+  if (a->residual && a->res_dtype != EVLM_BF16 && a->res_dtype != EVLM_F32) return EVLM_EINVAL;
+  {
+    const int rc_skinny = gemm_skinny_try(a, a_scale, b_scale, stream);
+    if (rc_skinny != -1) return rc_skinny;
+  }
+  return gemm_tcgen05_run(a, a_scale, b_scale, stream);
+}
+
+// The tcgen05 path of evlm_gemm_bf16 (a_scale == nullptr) and evlm_gemm_fp8 (e4m3 operands, validated by the caller).
+static int evlm::gemm_tcgen05_run(const evlm_gemm_args* a, const float* a_scale, const float* b_scale, void* stream) {
+  const bool f8 = a_scale != nullptr;
+  const int bk = f8 ? BLOCK_K_F8 : BLOCK_K;
   const int epi = a->epi_mode == EVLM_EPI_ACT_BACKWARD ? EPI_ACT_BWD
                   : (a->act != EVLM_ACT_NONE || a->gate_mode != EVLM_GATE_NONE) ? EPI_ACT_FWD : EPI_LINEAR;
 
@@ -918,9 +988,11 @@ extern "C" int evlm_gemm_bf16(const evlm_gemm_args* a, void* stream) {
 
   GemmParams p;
   p.g = *a;
+  p.a_scale = a_scale;
+  p.b_scale = b_scale;
   p.m_tiles = m_tiles;
   p.n_tiles = (a->N + block_n - 1) / block_n;
-  p.k_blocks = (a->K + BLOCK_K - 1) / BLOCK_K;
+  p.k_blocks = (a->K + bk - 1) / bk;
   {
     int sp = a->splits > 1 ? (a->splits < p.k_blocks ? a->splits : p.k_blocks) : 1;
     p.kb_per_split = (p.k_blocks + sp - 1) / sp;
@@ -929,12 +1001,19 @@ extern "C" int evlm_gemm_bf16(const evlm_gemm_args* a, void* stream) {
   p.g.splits = p.splits;
 
   int rc;
-  if (!a->a_mn) rc = make_tmap_bf16(&p.tma_a, a->A, a->M, a->K, a->lda, BLOCK_M);
-  else          rc = make_tmap_bf16(&p.tma_a, a->A, a->K, a->M, a->lda, BLOCK_K);
-  if (rc) return rc;
-  if (!a->b_mn) rc = make_tmap_bf16(&p.tma_b, a->B, a->N, a->K, a->ldb, block_n);
-  else          rc = make_tmap_bf16(&p.tma_b, a->B, a->K, a->N, a->ldb, BLOCK_K);
-  if (rc) return rc;
+  if (f8) {   // (K-major only)
+    rc = make_tmap_e4m3(&p.tma_a, a->A, a->M, a->K, a->lda, BLOCK_M);
+    if (rc) return rc;
+    rc = make_tmap_e4m3(&p.tma_b, a->B, a->N, a->K, a->ldb, block_n);
+    if (rc) return rc;
+  } else {
+    if (!a->a_mn) rc = make_tmap_bf16(&p.tma_a, a->A, a->M, a->K, a->lda, BLOCK_M);
+    else          rc = make_tmap_bf16(&p.tma_a, a->A, a->K, a->M, a->lda, BLOCK_K);
+    if (rc) return rc;
+    if (!a->b_mn) rc = make_tmap_bf16(&p.tma_b, a->B, a->N, a->K, a->ldb, block_n);
+    else          rc = make_tmap_bf16(&p.tma_b, a->B, a->K, a->N, a->ldb, BLOCK_K);
+    if (rc) return rc;
+  }
 
   // epilogue stores through TMA whenever base and row pitch are 16-byte multiples (everything the host side allocates is)
   p.tma_d_ok = p.tma_aux_ok = 0;
@@ -980,6 +1059,7 @@ extern "C" int evlm_gemm_bf16(const evlm_gemm_args* a, void* stream) {
   const int64_t total = (int64_t)p.m_tiles * p.n_tiles * p.splits;
   const int grid = (int)(total < sms ? total : sms);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  if (f8) return block_n == 256 ? dispatch_f8<256>(p, grid, st, epi, db) : dispatch_f8<128>(p, grid, st, epi, db);
   return block_n == 256 ? dispatch<256>(p, grid, st, a->a_mn, a->b_mn, epi, db) : dispatch<128>(p, grid, st, a->a_mn, a->b_mn, epi, db);
 }
 

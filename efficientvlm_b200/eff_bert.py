@@ -170,6 +170,8 @@ def _key_mask_from_ext(mask):
 
 
 class BertLayer(nn.Module):
+    evlm_fp8 = False      # set by fp8.enable: every projection of the layer runs in e4m3 (inference only)
+
     def __init__(self, config, layer_num):
         super().__init__()
         self.config = config
@@ -208,7 +210,7 @@ class BertLayer(nn.Module):
         cfg = ops.LayerCfg(sa.num_attention_heads, self.output.LayerNorm.eps, want_probs=bool(output_attentions), training=self.training,
                            attn_dropout=sa.dropout.p, hidden_dropout=self.output.dropout.p, causal=causal,
                            has_cross=self.has_cross_attention,
-                           cross_heads=self.crossattention.self.num_attention_heads if self.has_cross_attention else 0)
+                           cross_heads=self.crossattention.self.num_attention_heads if self.has_cross_attention else 0, fp8=self.evlm_fp8)
         params = self.attention._params()
         if self.has_cross_attention:
             params = params + self.crossattention._params()
@@ -314,17 +316,21 @@ class BertPooler(nn.Module):
 
 
 class BertPredictionHeadTransform(nn.Module):
+    evlm_fp8 = False      # set by fp8.enable
+
     def __init__(self, config):
         super().__init__()
         self.dense = nn.Linear(config.hidden_size, config.hidden_size)
         self.LayerNorm = nn.LayerNorm(config.hidden_size, eps=config.layer_norm_eps)
 
     def forward(self, hidden_states):
-        h = ops.linear(hidden_states, self.dense.weight, self.dense.bias, act=ACT_GELU_ERF)
+        h = (ops.linear_fp8 if self.evlm_fp8 else ops.linear)(hidden_states, self.dense.weight, self.dense.bias, act=ACT_GELU_ERF)
         return ops.layer_norm(h, self.LayerNorm.weight, self.LayerNorm.bias, self.LayerNorm.eps)
 
 
 class BertLMPredictionHead(nn.Module):
+    evlm_fp8 = False      # set by fp8.enable: the (tied) vocabulary product runs in e4m3
+
     def __init__(self, config):
         super().__init__()
         self.transform = BertPredictionHeadTransform(config)
@@ -333,7 +339,7 @@ class BertLMPredictionHead(nn.Module):
         self.decoder.bias = self.bias  # same Parameter under two state_dict names (eff_bert.py:738-741)
 
     def forward(self, hidden_states):
-        return ops.linear(self.transform(hidden_states), self.decoder.weight, self.bias)
+        return (ops.linear_fp8 if self.evlm_fp8 else ops.linear)(self.transform(hidden_states), self.decoder.weight, self.bias)
 
 
 class BertOnlyMLMHead(nn.Module):

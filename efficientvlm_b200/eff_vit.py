@@ -88,6 +88,8 @@ class CLIPMLP(nn.Module):
 
 
 class CLIPEncoderLayer(nn.Module):
+    evlm_fp8 = False      # set by fp8.enable: the four projections run in e4m3 (inference only)
+
     def __init__(self, hidden_size, hidden_act, num_attention_heads, attention_dropout, intermediate_size):
         super().__init__()
         self.self_attn = CLIPAttention(hidden_size, num_attention_heads, attention_dropout)
@@ -117,7 +119,7 @@ class CLIPEncoderLayer(nn.Module):
             key_mask = key_mask.to(torch.float32).contiguous()
         a = self.self_attn
         cfg = ops.LayerCfg(a.num_heads, self.layer_norm1.eps, want_probs=bool(output_attentions), training=self.training,
-                           attn_dropout=a.dropout)
+                           attn_dropout=a.dropout, fp8=self.evlm_fp8)
         out, probs = ops.vit_layer(hidden_states, key_mask, head_z, head_layer_z, mlp_z, cfg, self._params())
         outputs = (out,)
         if output_attentions:

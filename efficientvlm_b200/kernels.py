@@ -102,6 +102,48 @@ def gemm(A, B, D, M, N, K, *, a_mn=False, b_mn=False, epi_mode=0, bias=None, alp
     return D
 
 
+e4m3 = torch.float8_e4m3fn
+
+
+def quant_rows_e4m3(x, out=None, scale=None):
+    """Rows of x (bf16 / fp32 [R, K], any row pitch) -> (q e4m3 [R, K] view of a [R, ldq] buffer with ldq % 16 == 0 and zero pad bytes,
+    scale fp32 [R]).  q = satfinite_rn(x * (448 / amax_row)), scale = amax_row / 448 (include/evlm.h)."""
+    assert x.dim() == 2 and x.stride(1) == 1
+    R, Kd = x.shape
+    if out is None:
+        out = torch.empty(R, (Kd + 15) // 16 * 16, dtype=e4m3, device=x.device)[:, :Kd]
+    if scale is None:
+        scale = torch.empty(R, dtype=f32, device=x.device)
+    assert out.dtype == e4m3 and out.shape == (R, Kd) and out.stride(1) == 1 and scale.dtype == f32 and scale.numel() == R
+    check(_lib.load().evlm_quant_rows_e4m3(_p(x), _dt(x), x.stride(0), R, Kd, _p(out), out.stride(0), _p(scale), _stream()),
+          "evlm_quant_rows_e4m3")
+    return out, scale
+
+
+def gemm_fp8(A, a_scale, B, b_scale, D, M, N, K, *, bias=None, alpha=1.0, alpha_cols=0, act=0, aux_out=None, residual=None):
+    """D[M,N] = epilogue(a_scale[m] b_scale[n] sum_k A[m,k] B[n,k]); A / B e4m3 [rows, K] views with 16-byte row pitches (as
+    quant_rows_e4m3 leaves them).  The forward epilogue of gemm() without gates, dropout, splits or limits."""
+    assert A.dtype == e4m3 and B.dtype == e4m3 and A.dim() == 2 and B.dim() == 2 and D.dim() == 2
+    assert A.stride(1) == 1 and B.stride(1) == 1 and D.stride(1) == 1
+    assert a_scale.dtype == f32 and b_scale.dtype == f32
+    g = GemmArgs()
+    g.M, g.N, g.K = M, N, K
+    g.A, g.lda = _p(A), A.stride(0)
+    g.B, g.ldb = _p(B), B.stride(0)
+    g.D, g.ldd, g.d_dtype = _p(D), D.stride(0), _dt(D)
+    g.bias = _p(bias)
+    g.alpha, g.alpha_cols = alpha, alpha_cols
+    g.act = act
+    if aux_out is not None:
+        g.aux_out, g.ld_aux_out = _p(aux_out), aux_out.stride(0)
+    if residual is not None:
+        assert residual.dim() == 2 and residual.stride(1) == 1
+        g.residual, g.ldr, g.res_dtype = _p(residual), residual.stride(0), _dt(residual)
+    g.splits, g.max_ctas = 1, GEMM_MAX_CTAS
+    check(_lib.load().evlm_gemm_fp8(C.byref(g), _p(a_scale), _p(b_scale), _stream()), "evlm_gemm_fp8")
+    return D
+
+
 GEMM_PROFILE = None
 GEMM_MAX_CTAS = 0      # persistent-grid width of the tcgen05 GEMM (0 = every SM); profiling knob
 HBM_PROFILE = None      # bench.py: list of (kernel name, start event, end event, algorithmic bytes) for the HBM-bound kernels

@@ -37,6 +37,7 @@ def next_seed():
 # bf16 weight shadows
 # ----------------------------------------------------------------------------------------------------------------------
 _w16 = {}
+_w8 = {}
 _cat = {}
 _epoch = [0]
 _pepoch = {}
@@ -55,6 +56,7 @@ def invalidate_weight_cache(params=None):
 
 def clear_weight_cache():
     _w16.clear()
+    _w8.clear()
     _cat.clear()
 
 
@@ -106,6 +108,68 @@ def weight_bf16(*ws):
             del _w16[k]
     _w16[key] = (ver, out, tuple(weakref.ref(w) for w in ws))
     return out
+
+
+class Fp8Weight:
+    """e4m3 shadow of one or several stacked fp32 weights [N, K]: q [N, K] (16-byte row pitch) and one fp32 scale per output channel."""
+    __slots__ = ("q", "scale")
+
+    def __init__(self, q, scale):
+        self.q, self.scale = q, scale
+
+    def data_ptr(self):
+        return self.q.data_ptr()
+
+
+def weight_e4m3(*ws):
+    """Fp8Weight of the fp32 weights `ws` stacked along dim 0, cached and invalidated exactly like weight_bf16.  Rows are quantised
+    independently (K.quant_rows_e4m3, one launch per weight), so the stacked shadow equals the quantisation of the stacked matrix."""
+    key = tuple(id(w) for w in ws)
+    ver = (tuple((w._version, w.data_ptr(), _pepoch.get(id(w), 0)) for w in ws), _epoch[0])
+    ent = _w8.get(key)
+    alive = ent is not None and all(r() is w for r, w in zip(ent[2], ws))
+    if alive and ent[0] == ver:
+        return ent[1]
+    rows = sum(w.shape[0] for w in ws)
+    cols = ws[0][0].numel()
+    out = Fp8Weight(torch.empty(rows, (cols + 15) // 16 * 16, dtype=K.e4m3, device=ws[0].device)[:, :cols],
+                    torch.empty(rows, dtype=f32, device=ws[0].device))
+    r = 0
+    for w in ws:
+        if w.shape[0]:
+            K.quant_rows_e4m3(w.detach().reshape(w.shape[0], cols), out.q[r:r + w.shape[0]], out.scale[r:r + w.shape[0]])
+        r += w.shape[0]
+    if len(_w8) > 4096:
+        for k in [k for k, e in _w8.items() if any(rf() is None for rf in e[2])]:
+            del _w8[k]
+    _w8[key] = (ver, out, tuple(weakref.ref(w) for w in ws))
+    return out
+
+
+def weight_fwd(fp8, *ws):
+    """The forward operand of a covered Linear: the bf16 shadow, or the e4m3 one when the layer runs FP8 inference (fp8.enable)."""
+    return weight_e4m3(*ws) if fp8 else weight_bf16(*ws)
+
+
+def gemm_fwd(a16, W, D, M, N, Kd, dropout_p=0.0, seed=0, stream_id=0, gate=None, gate_mode=0, **epi):
+    """Forward product D = epilogue(a16 W^T) of a covered Linear with the operand weight_fwd returned.  bf16: K.gemm.  FP8: the bf16
+    activation is quantised per row (K.quant_rows_e4m3) and multiplied by the e4m3 weight (K.gemm_fp8); the epilogue is the same."""
+    if not isinstance(W, Fp8Weight):
+        return K.gemm(a16, W, D, M, N, Kd, dropout_p=dropout_p, seed=seed, stream_id=stream_id, gate=gate, gate_mode=gate_mode, **epi)
+    if dropout_p > 0.0 or gate is not None:
+        raise ValueError("FP8 inference has no dropout and no gates (it runs a model that prune.materialize has pruned, in eval mode)")
+    qa, sa = K.quant_rows_e4m3(a16)
+    return K.gemm_fp8(qa, sa, W.q, W.scale, D, M, N, Kd, **epi)
+
+
+def _fp8_inference_only(fp8, training, need_grad, *gates):
+    if not fp8:
+        return
+    if training or need_grad:
+        raise RuntimeError("efficientvlm_b200: this model runs FP8 inference (fp8.enable), which has no backward: call it in eval mode "
+                           "under torch.no_grad() / torch.inference_mode()")
+    if any(z is not None for z in gates):
+        raise ValueError("efficientvlm_b200: FP8 inference runs without gates (the gates of a materialised model live in its weights)")
 
 
 _refresh_tables = {}
@@ -557,7 +621,7 @@ class LayerCfg:
     """Static (non-tensor) configuration of one transformer layer call."""
 
     def __init__(self, num_heads, eps, want_probs=False, training=False, attn_dropout=0.0, hidden_dropout=0.0, causal=False,
-                 has_cross=False, cross_heads=0, past_len=0, fp16_prescale=False):
+                 has_cross=False, cross_heads=0, past_len=0, fp16_prescale=False, fp8=False):
         self.num_heads = num_heads
         self.eps = eps
         self.want_probs = want_probs
@@ -569,6 +633,7 @@ class LayerCfg:
         self.cross_heads = cross_heads
         self.past_len = past_len
         self.fp16_prescale = fp16_prescale
+        self.fp8 = fp8                 # forward products in e4m3 (fp8.enable): inference only
 
 
 # ----------------------------------------------------------------------------------------------------------------------
@@ -616,24 +681,25 @@ class VitLayerFn(torch.autograd.Function):
             raise ValueError("head_dim must be 64 (embed %d, heads %d)" % (E, nh))
         if head_layer_z is not None and _needs_grad(ctx):
             raise NotImplementedError("head_layer_z is forward-only (never produced by the reference's live L0 modules)")
+        _fp8_inference_only(cfg.fp8, cfg.training, _needs_grad(ctx), head_z, head_layer_z, mlp_z)
         x2 = h.contiguous().reshape(T, H)
         _, a16, mean1, rstd1 = K.layernorm_fwd(x2, ln1w, ln1b, cfg.eps, want_f32=False, want_bf16=True)
-        Wqkv = weight_bf16(qw, kw, vw)
+        Wqkv = weight_fwd(cfg.fp8, qw, kw, vw)
         qkv = alloc16(T, 3 * E, dev)
-        K.gemm(a16, Wqkv, qkv, T, 3 * E, H, bias=bias_cat(qb, kb, vb))
+        gemm_fwd(a16, Wqkv, qkv, T, 3 * E, H, bias=bias_cat(qb, kb, vb))
         hz = _flat_gate(head_z, nh)
         p_att = cfg.attn_dropout if cfg.training else 0.0
         seed = next_seed() if p_att > 0 else 0
         # (q W^T + b) * 64^-0.5 (eff_vit.py:137): the power-of-two scale commutes exactly with bf16 rounding
         c16, probs, lse = K.attention_fwd(qkv[:, :E], qkv[:, E:2 * E], qkv[:, 2 * E:], B, nh, N, N, 0.125, key_mask=key_mask, head_z=hz,
                                           want_probs=cfg.want_probs, dropout_p=p_att, seed=seed, stream_id=0)
-        Wo = weight_bf16(ow)
+        Wo = weight_fwd(cfg.fp8, ow)
         h1 = torch.empty(T, H, dtype=f32, device=dev)
         hlz = _flat_gate(head_layer_z.expand(1, 1, H) if head_layer_z is not None and head_layer_z.numel() == 1 else head_layer_z, H)
-        K.gemm(c16, Wo, h1, T, H, E, bias=ob.detach(), gate=hlz, gate_mode=GATE_POST_ACT, residual=x2)
+        gemm_fwd(c16, Wo, h1, T, H, E, bias=ob.detach(), gate=hlz, gate_mode=GATE_POST_ACT, residual=x2)
         _, m16, mean2, rstd2 = K.layernorm_fwd(h1, ln2w, ln2b, cfg.eps, want_f32=False, want_bf16=True)
-        W1 = weight_bf16(f1w)
-        W2 = weight_bf16(f2w)
+        W1 = weight_fwd(cfg.fp8, f1w)
+        W2 = weight_fwd(cfg.fp8, f2w)
         need_grad = _needs_grad(ctx)
         g16 = alloc16(T, I, dev)
         u16 = alloc16(T, I, dev) if need_grad else None
@@ -641,8 +707,8 @@ class VitLayerFn(torch.autograd.Function):
         cpk = _compact_for(mz, W1, f1w, f1b, W2, f2w) if getattr(cfg, "ffn_skip", False) else None
         h2 = torch.empty(T, H, dtype=f32, device=dev)
         if cpk is None:
-            K.gemm(m16, W1, g16, T, I, H, bias=f1b.detach(), act=ACT_QUICK_GELU, gate=mz, gate_mode=GATE_PRE_ACT, aux_out=u16)
-            K.gemm(g16, W2, h2, T, H, I, bias=f2b.detach(), residual=h1)
+            gemm_fwd(m16, W1, g16, T, I, H, bias=f1b.detach(), act=ACT_QUICK_GELU, gate=mz, gate_mode=GATE_PRE_ACT, aux_out=u16)
+            gemm_fwd(g16, W2, h2, T, H, I, bias=f2b.detach(), residual=h1)
         else:     # kept columns only (device-side limit)
             K.gemm(m16, cpk.W1, g16, T, I, H, bias=cpk.b1, act=ACT_QUICK_GELU, gate=cpk.z, gate_mode=GATE_PRE_ACT, aux_out=u16, n_limit=cpk.count)
             K.gemm(g16, cpk.W2, h2, T, H, I, bias=f2b.detach(), residual=h1, k_limit=cpk.count)
@@ -820,7 +886,7 @@ class LinearFn(torch.autograd.Function):
     """y = act(x W^T + b), fp32 in / fp32 out, bf16 tensor-core GEMM inside."""
 
     @staticmethod
-    def forward(ctx, x, w, b, act):
+    def forward(ctx, x, w, b, act, fp8):
         shape = x.shape
         Kin = shape[-1]
         Nout = w.shape[0]
@@ -829,13 +895,14 @@ class LinearFn(torch.autograd.Function):
         dev = x.device
         x16 = alloc16(M, Kin, dev)
         K.cast_bf16(x2, x16)
-        W16 = weight_bf16(w)
+        need = _needs_grad(ctx)
+        _fp8_inference_only(fp8, False, need)
+        W16 = weight_fwd(fp8, w)
         # row pitch padded to 16 bytes: the epilogue's TMA box stores need it (vocabulary 30522 -> pitch 30524; without it the
         # [1024, 30522] MLM logits fall back to scalar stores: 146 us instead of ~40 us per launch)
         y = torch.empty(M, Nout, dtype=f32, device=dev) if Nout % 4 == 0 else torch.empty(M, (Nout + 3) // 4 * 4, dtype=f32, device=dev)[:, :Nout]
-        need = _needs_grad(ctx)
         u16 = alloc16(M, Nout, dev) if (need and act != ACT_NONE) else None
-        K.gemm(x16, W16, y, M, Nout, Kin, bias=None if b is None else b.detach(), act=act, aux_out=u16)
+        gemm_fwd(x16, W16, y, M, Nout, Kin, bias=None if b is None else b.detach(), act=act, aux_out=u16)
         if need:
             ctx.saved = (x16, W16, u16)
             ctx.params = (w, b)
@@ -866,11 +933,16 @@ class LinearFn(torch.autograd.Function):
             dx = torch.empty(M, Kin, dtype=f32, device=dev)
             K.gemm(d16, W16, dx, M, Kin, Nout, b_mn=True)
             dx = dx.view(*dy.shape[:-1], Kin)
-        return dx, dW, db, None
+        return dx, dW, db, None, None
 
 
 def linear(x, w, b=None, act=ACT_NONE):
-    return _apply(LinearFn, x, w, b, act)
+    return _apply(LinearFn, x, w, b, act, False)
+
+
+def linear_fp8(x, w, b=None, act=ACT_NONE):
+    """linear() with the product in e4m3: the LM head of a model that fp8.enable has switched (inference only)."""
+    return _apply(LinearFn, x, w, b, act, True)
 
 
 class ActFn(torch.autograd.Function):
@@ -1011,6 +1083,7 @@ class BertLayerFn(torch.autograd.Function):
         need = _needs_grad(ctx)
         if need and past_k is not None:
             raise NotImplementedError("KV-cache decoding is inference-only")
+        _fp8_inference_only(cfg.fp8, cfg.training, need, shz, chz, mlp_z)
         train = cfg.training
         p_att = cfg.attn_dropout if train else 0.0
         p_hid = cfg.hidden_dropout if train else 0.0
@@ -1021,9 +1094,9 @@ class BertLayerFn(torch.autograd.Function):
         if x16 is None:
             x16 = K.cast_bf16(x2)
         # ---- self attention ----
-        Wqkv = weight_bf16(sp[0], sp[2], sp[4])
+        Wqkv = weight_fwd(cfg.fp8, sp[0], sp[2], sp[4])
         qkv = alloc16(T, 3 * E, dev)
-        K.gemm(x16, Wqkv, qkv, T, 3 * E, H, bias=bias_cat(sp[1], sp[3], sp[5]))
+        gemm_fwd(x16, Wqkv, qkv, T, 3 * E, H, bias=bias_cat(sp[1], sp[3], sp[5]))
         q, k, v = qkv[:, :E], qkv[:, E:2 * E], qkv[:, 2 * E:]
         Lk = L
         k_new, v_new = k, v
@@ -1054,9 +1127,9 @@ class BertLayerFn(torch.autograd.Function):
         c16, probs, lse = K.attention_fwd(q, k, v, B, nh, L, Lk, scale, key_mask=key_mask, causal=cfg.causal, causal_offset=Lk - L,
                                           head_z=hz, want_probs=cfg.want_probs, dropout_p=p_att, seed=seed, stream_id=0,
                                           pack_items=spack, pack_own_kv=spack is not None, kv_item_rows=kv_rows)
-        Wo = weight_bf16(sp[6])
+        Wo = weight_fwd(cfg.fp8, sp[6])
         s1 = torch.empty(T, H, dtype=f32, device=dev)
-        K.gemm(c16, Wo, s1, T, H, E, bias=sp[7].detach(), dropout_p=p_hid, seed=seed, stream_id=1, residual=x2)
+        gemm_fwd(c16, Wo, s1, T, H, E, bias=sp[7].detach(), dropout_p=p_hid, seed=seed, stream_id=1, residual=x2)
         h1_32, h1_16, mean_a, rstd_a = K.layernorm_fwd(s1, sp[8], sp[9], cfg.eps, want_f32=True, want_bf16=True)
         # ---- cross attention ----
         cross_saved = None
@@ -1084,10 +1157,10 @@ class BertLayerFn(torch.autograd.Function):
                 raise ValueError("encoder_batch_index must be int32 with one entry per text row")
             enc16_obj = act_bf16(enc) if (enc.dtype == f32 and enc.is_contiguous()) else K.cast_bf16(enc.contiguous().to(f32).view(Bn * Nn, He))
             enc16 = enc16_obj.view(Bn * Nn, He)       # a NEW tensor object every call: cache identity is checked on enc16_obj
-            Wq = weight_bf16(cp[0])
-            Wkv = weight_bf16(cp[2], cp[4])
+            Wq = weight_fwd(cfg.fp8, cp[0])
+            Wkv = weight_fwd(cfg.fp8, cp[2], cp[4])
             qx = alloc16(T, Ex, dev)
-            K.gemm(h1_16, Wq, qx, T, Ex, H, bias=cp[1].detach())
+            gemm_fwd(h1_16, Wq, qx, T, Ex, H, bias=cp[1].detach())
             # Inference (nothing saved for a backward): the K|V projection of the encoder states is the same at every step of a
             # decode loop and in both decoder passes of rank_answer — keep the last few (keyed by the bf16 activation copy, which
             # act_bf16 caches per tensor version, and by the weight shadow, which changes with every optimizer step).
@@ -1100,7 +1173,7 @@ class BertLayerFn(torch.autograd.Function):
                 kvx = hit[2]
             else:
                 kvx = alloc16(Bn * Nn, 2 * Ex, dev)
-                K.gemm(enc16, Wkv, kvx, Bn * Nn, 2 * Ex, He, bias=bias_cat(cp[3], cp[5]))
+                gemm_fwd(enc16, Wkv, kvx, Bn * Nn, 2 * Ex, He, bias=bias_cat(cp[3], cp[5]))
                 if kv_key is not None:
                     if len(_cross_kv) >= 8:
                         _cross_kv.clear()
@@ -1119,24 +1192,24 @@ class BertLayerFn(torch.autograd.Function):
             fold_index = enc_index
             if enc_pack is not None and need:
                 fold_index = enc_index.index_select(0, enc_pack[:, 0].long()).contiguous()
-            Wox = weight_bf16(cp[6])
+            Wox = weight_fwd(cfg.fp8, cp[6])
             s2 = torch.empty(T, H, dtype=f32, device=dev)
-            K.gemm(cx16, Wox, s2, T, H, Ex, bias=cp[7].detach(), dropout_p=p_hid, seed=seed, stream_id=2, residual=h1_32)
+            gemm_fwd(cx16, Wox, s2, T, H, Ex, bias=cp[7].detach(), dropout_p=p_hid, seed=seed, stream_id=2, residual=h1_32)
             h2_32, h2_16, mean_x, rstd_x = K.layernorm_fwd(s2, cp[8], cp[9], cfg.eps, want_f32=True, want_bf16=True)
             cross_saved = (enc16, Wq, Wkv, qx, kvx, cz, cx16, lse_x, probs_x, Wox, s2, mean_x, rstd_x, Nn, He, Ex, nhx, enc_mask, enc_index, Bn,
                            enc_pack, fold_index)
         # ---- FFN ----
         I = fp[0].shape[0]
-        W1 = weight_bf16(fp[0])
-        W2 = weight_bf16(fp[2])
+        W1 = weight_fwd(cfg.fp8, fp[0])
+        W2 = weight_fwd(cfg.fp8, fp[2])
         g16 = alloc16(T, I, dev)
         u16 = alloc16(T, I, dev) if need else None
         mz = _flat_gate(mlp_z, I)
         cpk = _compact_for(mz, W1, fp[0], fp[1], W2, fp[2]) if getattr(cfg, "ffn_skip", False) else None
         s3 = torch.empty(T, H, dtype=f32, device=dev)
         if cpk is None:
-            K.gemm(h2_16, W1, g16, T, I, H, bias=fp[1].detach(), act=ACT_GELU_ERF, gate=mz, gate_mode=GATE_POST_ACT, aux_out=u16)
-            K.gemm(g16, W2, s3, T, H, I, bias=fp[3].detach(), dropout_p=p_hid, seed=seed, stream_id=3, residual=h2_32)
+            gemm_fwd(h2_16, W1, g16, T, I, H, bias=fp[1].detach(), act=ACT_GELU_ERF, gate=mz, gate_mode=GATE_POST_ACT, aux_out=u16)
+            gemm_fwd(g16, W2, s3, T, H, I, bias=fp[3].detach(), dropout_p=p_hid, seed=seed, stream_id=3, residual=h2_32)
         else:     # kept columns only (device-side limit)
             K.gemm(h2_16, cpk.W1, g16, T, I, H, bias=cpk.b1, act=ACT_GELU_ERF, gate=cpk.z, gate_mode=GATE_POST_ACT, aux_out=u16, n_limit=cpk.count)
             K.gemm(g16, cpk.W2, s3, T, H, I, bias=fp[3].detach(), dropout_p=p_hid, seed=seed, stream_id=3, residual=h2_32, k_limit=cpk.count)

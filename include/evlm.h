@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define EVLM_ABI_VERSION 8
+#define EVLM_ABI_VERSION 9
 int evlm_abi_version(void);
 /* Number of kernel launches issued through this library by the calling process (bench gpu_launches). */
 unsigned long long evlm_launch_count(void);
@@ -75,6 +75,21 @@ typedef struct evlm_gemm_args {
 } evlm_gemm_args;
 
 int evlm_gemm_bf16(const evlm_gemm_args* args, void* stream);
+
+/* ABI v9 — FP8 inference (csrc/fp8.cu, the F8 instantiations of gemm_tcgen05.cu / gemm_skinny.cu).
+ * evlm_quant_rows_e4m3: rows of x [rows, cols] (x_dtype EVLM_BF16 | EVLM_F32, row pitch ldx elements) -> e4m3 q [rows, ldq bytes] and one
+ *   fp32 scale per row, with a fixed formula that a host mirror reproduces bit for bit:
+ *     amax = max_k |x[r,k]|;  inv = 448 / amax (IEEE division);  q[r,k] = cvt.rn.satfinite.e4m3(x[r,k] * inv);  scale[r] = amax / 448
+ *   (amax == 0: q = 0, scale = 0).  ldq % 16 == 0 and ldq >= cols (the TMA row pitch of the GEMM operands); bytes [cols, ldq) of every row
+ *   are written as 0.  One launch serves both operands: activations (a scale per token row) and weights [N, K] (a scale per output channel).
+ * evlm_gemm_fp8: D = epilogue(a_scale[m] * b_scale[n] * sum_k qa[m,k] * qb[n,k]) with A and B e4m3 (the pointers of args), both K-major,
+ *   lda / ldb in bytes, multiples of 16, bases 16-byte aligned.  The forward epilogue of evlm_gemm_args applies to the scaled accumulator:
+ *   bias, alpha q-scale, activation (quick-GELU / erf-GELU, optional aux_out), fp32 or bf16 residual, fp32 or bf16 D.  Everything else —
+ *   epi_mode != FORWARD, dropout, splits > 1, accumulate, gates, device-side limits, MN-major operands — returns EVLM_EINVAL.
+ *   M <= 32: weight-stream kernel (16-byte lane loads of 16 e4m3); otherwise tcgen05.mma.kind::f8f6f4 with 128-element k blocks. */
+int evlm_quant_rows_e4m3(const void* x, int32_t x_dtype, int64_t ldx, int64_t rows, int64_t cols, void* q, int64_t ldq, float* scale,
+                         void* stream);
+int evlm_gemm_fp8(const evlm_gemm_args* args, const float* a_scale, const float* b_scale, void* stream);
 
 /* fp32 SIMT contraction for the tiny, precision-critical products (ITC similarity xvlm.py:397-399 and
  * its backward): D[M,N] = alpha * A[M,K] * op(B) (+ beta*D), b_trans=1: B is [N,K]; 0: B is [K,N];
