@@ -271,6 +271,7 @@ class XVLM(XVLMBaseUngated):
 
 class EffXVLMforRetrieval(XVLMBase):
     """efficient_models/model_retrieval.py:7-92 — L0-gated ITR model."""
+    gates_folded = False        # set by prune.materialize: retrieval_eval.evaluation then runs without gates, forward refuses
 
     def __init__(self, config):
         super().__init__(config, load_vision_params=False, load_text_params=False, use_contrastive_loss=True, use_matching_loss=True,
@@ -283,6 +284,9 @@ class EffXVLMforRetrieval(XVLMBase):
         checkpoint.load_into(self, load_pretrained(ckpt_rpath, config, is_eval=is_eval, load_text=True), ckpt_rpath)
 
     def forward(self, image, text_ids, text_atts, idx=None, output_attentions=None, output_hidden_states=None):
+        if self.gates_folded:
+            raise RuntimeError("this retrieval model was materialised (prune.materialize): its gates are folded into pruned weights, so "
+                               "the training forward, which applies full-width gates, cannot run on it; use retrieval_eval.evaluation")
         kd = bool(output_attentions)
         zs = self.l0_module.forward(training=kd)                                # model_retrieval.py:26-27,78-79
         oa, oh = (output_attentions, output_hidden_states) if kd else (None, None)

@@ -32,6 +32,7 @@ def _nlvr_text_config(config):
 class XVLMForNLVR(XVLMBase):
     """models/model_nlvr.py:126-245 — un-gated NLVR2 model (the distillation teacher of Eff_NLVR.py)."""
     gated = False
+    gates_folded = False        # set by prune.materialize: the deterministic gates live in the (physically pruned) weights
 
     def __init__(self, config):
         config_text, num_text_layers, num_cross_layers = _nlvr_text_config(config)
@@ -68,7 +69,7 @@ class XVLMForNLVR(XVLMBase):
         checkpoint.load_into(self, state_dict, ckpt_rpath)
 
     def _gates(self, train):
-        if not self.gated:
+        if not self.gated or self.gates_folded:
             return dict(vision_head=None, vision_mlp=None, enc_head=None, enc_mlp=None)
         if train:
             zs = self.l0_module.forward(training=True)
@@ -80,7 +81,11 @@ class XVLMForNLVR(XVLMBase):
                     enc_mlp=torch.cat((zs["text_intermediate_z"], zs["cross_intermediate_z"]), dim=0))
 
     def forward(self, image, text_ids, text_atts, targets, train=True, output_attentions=None, output_hidden_states=None):
-        """image: [2B, 3, R, R] = the B first images followed by the B second images (model_nlvr.py:206-207)."""
+        """image: [2B, 3, R, R] = the B first images followed by the B second images (model_nlvr.py:206-207).
+        On a materialised model (prune.materialize) only the gate-free prediction `train=False` without KD outputs runs."""
+        if self.gates_folded and (train or output_attentions):
+            raise RuntimeError("this NLVR model was materialised (prune.materialize): its gates are folded into pruned weights, so the "
+                               "training and distillation forwards, which apply full-width gates, cannot run on it; use train=False")
         z = self._gates(train)
         n = targets.size(0)
         kd = bool(output_attentions)

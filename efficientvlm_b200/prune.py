@@ -18,12 +18,21 @@ head_z = cat(text_head_z, cross_head_z) and mlp_z = cat(text_intermediate_z, cro
 `eff_bert.layer_gate_rows` (quirk Q1: with fusion layer F, layer i >= F takes self row 2(i - F), cross row 2(i - F) + 1 and FFN row
 i - F, so the trailing cross_* rows are never read).  The reference's utils/caption_utils.py is not available, so parity with its
 captioning recipe is unpinned; the target is the gated model's own decode (tests/test_caption_materialize.py).
+
+NLVR2 models (`nlvr.XVLMForNLVR`): the text encoder runs in multi_modal mode with the same concatenated gates (nlvr.py `_gates`), so
+its text + 2 x cross layers take their rows through the same table (`concat_gate_rows`).  The reference's xvlm_utils.py folds the
+*intended* mapping for NLVR (text_head_z[i] / cross_head_z[2i]), not what its own gated forward applies; as for captioning, the target
+here is the gated model's own forward (tests/test_pruned_retrieval_nlvr.py).  The two per-image copies of a fusion layer share one
+cross-attention key / value parameter (`XVLMForNLVR.share_cross_attention`) but read different cross-head gate rows, so materialising
+first gives every copy its own key / value Linear: each copy then folds and prunes its own heads.  A materialised model is
+inference-only, so nothing needs the tie afterwards.
 """
 import torch
 
 from . import ops
 from .eff_bert import layer_gate_rows
 from .eff_vit import prune_linear_layer
+from .nlvr import XVLMForNLVR
 
 DIMS_PER_HEAD = 64
 
@@ -46,26 +55,50 @@ def _scale_value(att_self, head_z):
     att_self.value.bias.data = att_self.value.bias.data.mul(hz)
 
 
-def caption_decoder_gates(zs, decoder):
-    """Per decoder layer: (self head gate row, cross head gate row or None, FFN gate row), the rows the gated decoder of a captioning
-    model applies to that layer (see the module docstring)."""
+def concat_gate_rows(zs, bert):
+    """Per layer of `bert`: (self head gate row, cross head gate row or None, FFN gate row), the rows its gated multi_modal forward
+    applies to that layer with head_z = cat(text_head_z, cross_head_z) and mlp_z = cat(text_intermediate_z, cross_intermediate_z): the
+    decoder of a captioning model, the text encoder of an NLVR model (see the module docstring)."""
     heads = _rows(torch.cat((zs["text_head_z"], zs["cross_head_z"]), dim=0))
     mlps = _rows(torch.cat((zs["text_intermediate_z"], zs["cross_intermediate_z"]), dim=0))
     out = []
-    for i in range(len(decoder.encoder.layer)):
-        s, c, m = layer_gate_rows(i, decoder.encoder.fusion_layer)
+    for i in range(len(bert.encoder.layer)):
+        s, c, m = layer_gate_rows(i, bert.encoder.fusion_layer)
         out.append((heads[s], None if c is None else heads[c], mlps[m]))
     return out
 
 
-def _caption_plan(gates):
-    """Per decoder layer: (self heads to prune, cross heads to prune or None, FFN columns to keep); refuses a layer left empty."""
-    return [(_zero_heads(s, "decoder self", i), None if c is None else _zero_heads(c, "decoder cross", i), _kept_columns(m, "decoder", i))
+caption_decoder_gates = concat_gate_rows        # the name the captioning code and tests know it by
+
+
+def _concat_plan(gates, what):
+    """Per layer: (self heads to prune, cross heads to prune or None, FFN columns to keep); refuses a layer left empty."""
+    return [(_zero_heads(s, what + " self", i), None if c is None else _zero_heads(c, what + " cross", i), _kept_columns(m, what, i))
             for i, (s, c, m) in enumerate(gates)]
 
 
-def _is_captioner(model, zs):
-    return _bert_of(model, "text_encoder") is None and _bert_of(model, "text_decoder") is not None and "text_head_z" in zs
+def _concat_bert(model, zs):
+    """(BERT whose gates are the concatenated rows of `concat_gate_rows`, its name in errors), or (None, None) for the other models."""
+    if "text_head_z" not in zs:
+        return None, None
+    if _bert_of(model, "text_encoder") is None and _bert_of(model, "text_decoder") is not None:
+        return _bert_of(model, "text_decoder"), "decoder"
+    if isinstance(model, XVLMForNLVR):
+        return _bert_of(model, "text_encoder"), "encoder"
+    return None, None
+
+
+def _untie_cross_kv(bert):
+    """Every cross-attention layer gets its own copy of its key / value Linear (undoes XVLMForNLVR.share_cross_attention)."""
+    for blk in bert.encoder.layer:
+        if blk.has_cross_attention:
+            s = blk.crossattention.self
+            for name in ("key", "value"):
+                lin = getattr(s, name)
+                own = torch.nn.Linear(lin.in_features, lin.out_features, device=lin.weight.device, dtype=lin.weight.dtype)
+                own.weight.copy_(lin.weight)
+                own.bias.copy_(lin.bias)
+                setattr(s, name, own)
 
 
 @torch.no_grad()
@@ -74,10 +107,17 @@ def update_params(model, zs):
     vision = model.vision_encoder
     text = _bert_of(model, "text_encoder")
     decoder = _bert_of(model, "text_decoder")
-    if _is_captioner(model, zs):
-        gates = caption_decoder_gates(zs, decoder)
-        _caption_plan(gates)                  # a layer that would be left empty is refused before any weight changes
-        for blk, (self_z, cross_z, mlp_z) in zip(decoder.encoder.layer, gates):
+    bert, what = _concat_bert(model, zs)
+    if bert is not None:
+        gates = concat_gate_rows(zs, bert)
+        _concat_plan(gates, what)             # a layer that would be left empty is refused before any weight changes
+        if "vision_head_z" in zs:
+            _heads_to_prune(zs["vision_head_z"], "vision")
+        if "vision_intermediate_z" in zs:
+            _kept_dims(zs["vision_intermediate_z"], "vision")
+        if what == "encoder":
+            _untie_cross_kv(bert)
+        for blk, (self_z, cross_z, mlp_z) in zip(bert.encoder.layer, gates):
             _scale_value(blk.attention.self, self_z)
             if cross_z is not None:
                 _scale_value(blk.crossattention.self, cross_z)
@@ -174,13 +214,14 @@ def prune_model_with_z(zs, model):
     vision = model.vision_encoder
     text = _bert_of(model, "text_encoder")
     decoder = _bert_of(model, "text_decoder")
-    if _is_captioner(model, zs):
-        plan = _caption_plan(caption_decoder_gates(zs, decoder))
-        for blk, (self_heads, cross_heads, _) in zip(decoder.encoder.layer, plan):
+    bert, what = _concat_bert(model, zs)
+    if bert is not None:
+        plan = _concat_plan(concat_gate_rows(zs, bert), what)
+        for blk, (self_heads, cross_heads, _) in zip(bert.encoder.layer, plan):
             blk.attention.prune_heads(self_heads)
             if cross_heads is not None:
                 blk.crossattention.prune_heads(cross_heads)
-        prune_intermediate_layers(decoder, {i: keep for i, (_, _, keep) in enumerate(plan)})
+        prune_intermediate_layers(bert, {i: keep for i, (_, _, keep) in enumerate(plan)})
         zs = {k: v for k, v in zs.items() if k.startswith("vision_")}
     if "vision_head_z" in zs:
         vision.prune_heads(_heads_to_prune(zs["vision_head_z"], "vision"))
@@ -205,7 +246,9 @@ def materialize(model, zs=None):
     """update_params + prune_model_with_z with the model's own deterministic masks (l0_module.forward(training=False)) by
     default.  Returns the per-module sizes `l0_module.calculate_model_size` reports.  The pruned model is then run WITHOUT gates
     (the reference's `fake_forward`, model_generation.py:214-230): see `efficientvlm_b200.vqa.XVLMForVQA.forward(..., use_gates=False)`.
-    Sets `model.gates_folded`: a captioning model's `generate` then runs without gates, and its `forward` refuses to run."""
+    Sets `model.gates_folded`: a captioning model's `generate`, an NLVR model's `forward(train=False)` and a retrieval model's
+    `retrieval_eval.evaluation` then run without gates, and the training forwards refuse to run.  A layer that would be left without
+    heads or FFN columns raises NotImplementedError; for captioning and NLVR models that happens before any weight changes."""
     if zs is None:
         with torch.no_grad():
             zs = model.l0_module.forward(training=False)

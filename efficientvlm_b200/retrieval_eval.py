@@ -144,13 +144,17 @@ def rerank_scores(model, image_feats, text_feats, text_atts, sims_matrix, k_test
 @torch.no_grad()
 def evaluation(model, data_loader, tokenizer, device, config, queries_per_pass=None, kv_cache_bytes=64 << 30, details=None, group_rows=16):
     """`Eff_Retrieval.py:216-332`.  Returns (score_matrix_i2t ndarray, score_matrix_t2i ndarray, pruned_model_sparsity).
-    `details` (optional dict) receives the intermediate tensors (sims_matrix, image_feats, text_feats, text_atts, zs)."""
+    `details` (optional dict) receives the intermediate tensors (sims_matrix, image_feats, text_feats, text_atts, zs).
+    On a materialised model (prune.materialize: its gates live in the pruned weights) every encoder and the re-rank run without gates;
+    the sparsity is still that of the deterministic masks, which materialize leaves in `l0_module`."""
     model.eval()
     texts = data_loader.dataset.text
     num_text = len(texts)
     text_bs = config["batch_size_test_text"]
     zs = model.l0_module.forward(training=False)
     pruned_model_size_info = model.l0_module.calculate_model_size(zs)
+    if getattr(model, "gates_folded", False):
+        zs = {k: None for k in zs}
     text_feats, text_embeds, text_atts = [], [], []
     for i in range(0, num_text, text_bs):
         text_input = tokenizer(texts[i:min(num_text, i + text_bs)], padding="max_length", truncation=True, max_length=config["max_tokens"],
